@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark contract of the B200-native NeRF hot path.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 One "step" = one full NeRF training iteration (BASELINE.json configs[1]: 800x800 synthetic Lego-shaped views,
 4096-ray batch per GPU, 64 coarse + 128 fine samples, fp16 tensor-core MLP with fp32 accumulate, Adam step
@@ -308,10 +308,13 @@ def run_gpu_arm(args) -> None:
         start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         start.record()
         for i in range(args.steps):
-            trainer.fused_step(batches[i % len(batches)], camera)
+            loss = trainer.fused_step(batches[i % len(batches)], camera)
         end.record()
         sync_all()
         elapsed_ms = start.elapsed_time(end)
+        # the regions below keep training, so what the last timed step returned (the loss in the step's static buffer)
+        # and left in the model (its parameters) is copied now
+        dumped = {'loss': loss.clone(), **{k: p.detach().clone() for k, p in model.named_parameters()}} if args.dump_outputs else None
         # ---- timed region B (end to end): pinned host buffers -> H2D copy every step, loss read back every step ----
         host = []
         for b in batches[:8]:
@@ -489,7 +492,21 @@ def run_gpu_arm(args) -> None:
                    'tensor_frac_of_burst_peak_per_gpu': render_tflops / world / peaks['bf16_tflops'], 'clocks': render_clocks.summary()},
         'stress': stress,
     }), flush=True)
+    if dumped is not None:
+        dump_outputs(Path(args.dump_outputs), dumped)
     _leave(world)
+
+
+def dump_outputs(out_dir: Path, arrays: dict[str, torch.Tensor]) -> None:
+    """Writes every array as out_dir/<name>.npy in float32, so that two builds run with the same arguments (hence the
+    same seeded inputs) can be compared output for output."""
+    import numpy as np
+    host = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    assert total <= 64 << 20, f'{total} bytes of outputs exceed the 64 MB dump budget'
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in host.items():
+        np.save(out_dir / f'{name}.npy', a)
 
 
 def _leave(world: int) -> None:
@@ -513,7 +530,14 @@ def main() -> None:
     ap.add_argument('--deadline', type=float, default=900.0,
                     help='seconds after which a run that is still going dumps every thread\'s stack to stderr and exits 1 '
                          '(a rank stuck in a collective must not hold a multi-GPU box until the caller\'s own limit)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one computed (its loss and the updated model parameters) '
+                         'as DIR/<name>.npy (float32; rank 0)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of the CUDA training step (--impl ours)')
     if args.deadline > 0:
         import faulthandler
         faulthandler.dump_traceback_later(args.deadline, exit=True)

@@ -79,7 +79,8 @@ def _worker(rank: int, world: int, port: int, out) -> None:
 
 def test_allreduce_mean_and_sharding_world2():
     world = 2
-    mgr = mp.Manager()
+    # the result server is spawned, not forked: earlier tests in the same process may have initialised CUDA and its threads
+    mgr = mp.get_context('spawn').Manager()
     out = mgr.dict()
     mp.spawn(_worker, args=(world, _free_port(), out), nprocs=world, join=True)
     assert dict(out) == {0: True, 1: True}
