@@ -10,10 +10,7 @@
 
 namespace nerf {
 
-#ifndef NERF_RAYS_PER_BLOCK
-#define NERF_RAYS_PER_BLOCK 4  // measured: 4, 8 and 16 rays per block time the same at config E (+-2 %)
-#endif
-constexpr int kRaysPerBlock = NERF_RAYS_PER_BLOCK;
+constexpr int kRaysPerBlock = 4;  // measured: 4, 8 and 16 rays per block time the same at config E (+-2 %)
 constexpr float kFinalDelta = 1.0e10f;
 constexpr int kMaxChunks = 64;  // S <= 2048
 

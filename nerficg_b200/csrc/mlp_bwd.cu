@@ -20,10 +20,7 @@ using namespace tc;
 namespace bwd {
 constexpr int kEpiThreadsPerSlot = 256;  // 8 warps per slot: 4 TMEM lane quarters x 2 column halves (mlp_fwd.cu)
 constexpr int kThreads = 128 + 2 * kEpiThreadsPerSlot;
-#ifndef NERF_BWD_RING
-#define NERF_BWD_RING 6
-#endif
-constexpr int kRingStages = NERF_BWD_RING;                           // 16 KB stages: this CTA's 128-column half of one W^T panel (mlp_fwd.cu)
+constexpr int kRingStages = 6;                                       // 16 KB stages: this CTA's 128-column half of one W^T panel (mlp_fwd.cu)
 constexpr uint32_t kRingStageBytes = kPanelBytes128;
 constexpr uint32_t kSlotBytes = kActBytes;
 constexpr uint32_t kOffRing = 2 * kSlotBytes;
@@ -31,20 +28,6 @@ constexpr uint32_t kOffBars = kOffRing + kRingStages * kRingStageBytes;
 constexpr uint32_t kSmemBytes = kOffBars + 256 + 1024;
 static_assert(kSmemBytes <= 232448, "shared memory budget exceeded");
 constexpr int kRegsEpilogue = 112, kRegsOther = 32;
-#if defined(NERF_NO_SHARE_W)
-constexpr bool kShareW = false;
-#else
-constexpr bool kShareW = true;   // one weight load per stage for both slots (mlp_fwd.cu); every dgrad stage fits the ring
-#endif
-#ifndef NERF_EXP_CPASYNC_MODE
-#define NERF_EXP_CPASYNC_MODE 0
-#endif
-constexpr uint32_t kLsuLag = 2;
-#if defined(NERF_EXP_CPASYNC_W) || defined(NERF_EXP_CPASYNC_W_ALL)
-constexpr bool kLsuW = true;    // weight ring filled by LSU cp.async instead of bulk copies (mlp_fwd.cu, DESIGN.md 4a fact 3)
-#else
-constexpr bool kLsuW = false;
-#endif
 // setmaxnreg moves registers inside the CTA's OWN allocation (launch: 640 threads x 96): what the 128 producer / MMA threads
 // release (96 - 32 each = 8192) must cover what the 512 epilogue threads request (112 - 96 each = 8192), or the
 // increase blocks forever
@@ -113,7 +96,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(bwd::kThreads, 1) ml
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (threadIdx.x == 0) {
     for (int i = 0; i < kRingStages; ++i) {
-      mbar_init(bar_w_full + 8 * i, (kLsuW && NERF_EXP_CPASYNC_MODE != 2) ? 32 : 1);   // LSU ring (mlp_fwd.cu): one cp.async-completion arrival per producer lane
+      mbar_init(bar_w_full + 8 * i, 1);
       mbar_init(bar_w_empty + 8 * i, 1);
       mbar_init(bar_w_peer + 8 * i, 1);
     }
@@ -148,9 +131,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(bwd::kThreads, 1) ml
     if (warp == 0) {
       // weight producer: rows [128 * rank, +128) (output columns of dX) of every W^T panel -> one ring stage
       uint32_t stage = 0, phase = 0;
-      uint32_t lsu_issued = 0, lsu_sig = 0;
-      (void)lsu_issued;
-      (void)lsu_sig;
       const uint64_t keep = l2_evict_last();
       long long t_wait = 0;
       const long long t_begin = prof_on ? clock64() : 0;
@@ -158,28 +138,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(bwd::kThreads, 1) ml
         for (int st = 0; st < kBwdStages; ++st)
           for (int slot = 0; slot < 2; ++slot) {
             if (!active(it, slot)) continue;
-            if (kShareW && slot == 1) continue;   // slot 1 re-uses the panels loaded for slot 0
+            if (slot == 1) continue;   // one weight load per stage for both slots (mlp_fwd.cu); every dgrad stage fits the ring
             const int first = bwd_first_panel(st), np = bwd_panels(st);
             for (int pp = 0; pp < np; ++pp) {
               NERF_TIMED(prof_on, t_wait, mbar_wait(bar_w_empty + 8 * stage, phase ^ 1));
-              if (kLsuW) {
-                const uint8_t* src = wimg + (uint32_t)(first + pp) * kPanelBytes256 + rank * kRingStageBytes + lane * 16;
-                const uint32_t dst = smem_base + kOffRing + stage * kRingStageBytes + lane * 16;
-#pragma unroll 8
-                for (uint32_t off = 0; off < kRingStageBytes; off += 512) cp_async16(dst + off, src + off);
-#if NERF_EXP_CPASYNC_MODE == 2
-                cp_async_commit();
-                if (++lsu_issued > kLsuLag) {
-                  cp_async_wait<kLsuLag>();
-                  fence_proxy_async_smem();
-                  __syncwarp();
-                  if (lane == 0) mbar_arrive(bar_w_full + 8 * lsu_sig);
-                  if (++lsu_sig == kRingStages) lsu_sig = 0;
-                }
-#else
-                cp_async_mbar_arrive_noinc(bar_w_full + 8 * stage);
-#endif
-              } else if (elect_one()) {
+              if (elect_one()) {
                 mbar_arrive_expect_tx(bar_w_full + 8 * stage, kRingStageBytes);
                 bulk_g2s_hint(smem_base + kOffRing + stage * kRingStageBytes,
                               wimg + (uint32_t)(first + pp) * kPanelBytes256 + rank * kRingStageBytes, kRingStageBytes,
@@ -192,18 +155,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(bwd::kThreads, 1) ml
               }
             }
           }
-#if NERF_EXP_CPASYNC_MODE == 2
-      if (kLsuW) {
-        cp_async_wait<0>();
-        fence_proxy_async_smem();
-        __syncwarp();
-        const uint32_t left = lsu_issued < kLsuLag ? lsu_issued : kLsuLag;
-        for (uint32_t i = 0; i < left; ++i) {
-          if (lane == 0) mbar_arrive(bar_w_full + 8 * lsu_sig);
-          if (++lsu_sig == kRingStages) lsu_sig = 0;
-        }
-      }
-#endif
       if (prof_on && lane == 0) {
         atomicAdd(p.prof + 13, (unsigned long long)t_wait);
         atomicAdd(p.prof + 14, (unsigned long long)(clock64() - t_begin));
@@ -221,11 +172,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(bwd::kThreads, 1) ml
           const uint32_t stage0 = stage, phase0 = phase;
           for (int slot = 0; slot < 2; ++slot) {
             if (!active(it, slot)) continue;
-            if (kShareW && slot == 1) {
+            if (slot == 1) {   // replay the ring stages slot 0 has just used (mlp_fwd.cu)
               stage = stage0;
               phase = phase0;
             }
-            const bool release = !kShareW || slot == 1 || !both;
+            const bool release = slot == 1 || !both;
             const uint32_t act = smem_base + slot * kSlotBytes;
             const uint32_t d_tmem = tmem_base + slot * 256;
             NERF_TIMED(prof_on, t_a, mbar_wait_cluster(bar_a_ready + 8 * slot, a_phase[slot]));
@@ -235,7 +186,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(bwd::kThreads, 1) ml
             for (int pp = 0; pp < np; ++pp) {
               NERF_TIMED(prof_on, t_w, mbar_wait(bar_w_full + 8 * stage, phase));
               NERF_TIMED(prof_on, t_w, mbar_wait_cluster(bar_w_peer + 8 * stage, phase));
-              if (kLsuW && NERF_EXP_CPASYNC_MODE != 2) fence_proxy_async_smem();
               tc_fence_after();
               if (elect_one()) {
                 const uint64_t da = make_smem_desc(act + pp * kPanelBytes128, 16u, kAtomBytes);
@@ -266,11 +216,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(bwd::kThreads, 1) ml
         for (int st = 0; st < kBwdStages; ++st)
           for (int slot = 0; slot < 2; ++slot) {
             if (!active(it, slot)) continue;
-            if (kShareW && slot == 1) continue;
+            if (slot == 1) continue;
             const int np = bwd_panels(st);
             for (int pp = 0; pp < np; ++pp) {
               mbar_wait(bar_w_full + 8 * stage, phase);
-              if (kLsuW && NERF_EXP_CPASYNC_MODE != 2) fence_proxy_async_smem();
               if (elect_one()) mbar_arrive_cluster(mapa(bar_w_peer + 8 * stage, 0));
               __syncwarp();
               if (++stage == kRingStages) {
@@ -311,21 +260,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(bwd::kThreads, 1) ml
 
       auto gstash_issue = [&](int region, uint32_t src, uint32_t bytes) {  // one thread, after the slot's warps fenced + met
         if (tg == 0 && tile_ok) {
-          #if defined(NERF_EXP_STORE_WRAP)   // diagnostic: every image lands in a 16-tile window that stays in L2 (results are wrong downstream)
-          const uint64_t tile_w = (uint64_t)(tile & 15);
-#else
-          const uint64_t tile_w = (uint64_t)tile;
-#endif
-          uint8_t* dst = p.gstash + grad_region_offset(region, n_tiles64) + tile_w * grad_region_tile_bytes(region);
-#if defined(NERF_EXP_NOSTORE)
-          (void)dst;
-#elif defined(NERF_EXP_SPLIT_STORE)
-          for (uint32_t off = 0; off < bytes; off += kPanelBytes128) bulk_s2g_hint(dst + off, src + off, kPanelBytes128, l2_evict_first());
-#elif defined(NERF_EXP_NOHINT)
-          bulk_s2g(dst, src, bytes);
-#else
+          uint8_t* dst = p.gstash + grad_region_offset(region, n_tiles64) + (uint64_t)tile * grad_region_tile_bytes(region);
           bulk_s2g_hint(dst, src, bytes, l2_evict_first());
-#endif
           bulk_commit();
         }
       };
@@ -474,16 +410,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(bwd::kThreads, 1) ml
           }
         };
         if (st == 1) run(BoolTag<true>{}); else run(BoolTag<false>{});
-#if defined(NERF_EXP_EARLY_HANDOFF)
-        fence_proxy_async_smem();
-        tc_fence_before();
-        if (st < kBwdStages - 1) {
-          __syncwarp();
-          if (lane == 0) mbar_arrive_cluster(a_ready_leader);
-        }
-        NERF_TIMED(prof, t_bar, named_bar_sync(bar_id, kEpiThreadsPerSlot));
-        gstash_issue(kGradF + st, act, kActBytes);
-#else
+        // operands are handed to the MMA issuer AFTER the slot's warps meet for the image store: the forward's early hand-off
+        // measured no faster here (dgrad 0.899 -> 0.900 ms, profiles/r02_store_path_variants.txt)
         gstash_store(kGradF + st, act, kActBytes);  // regions: F, L7, L6, ..., L0
         if (st < kBwdStages - 1) {
           fence_proxy_async_smem();
@@ -493,7 +421,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(bwd::kThreads, 1) ml
         } else {
           tc_fence_before();  // accumulator drained; released by the next tile's prologue arrive
         }
-#endif
       }
     }
     if (tg == 0) bulk_wait_all<0>();

@@ -586,20 +586,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(pipe::kThreads, 1) m
         PIPE_TIMED(e_acc, mbar_wait(bar_acc_ready, acc_phase));
         acc_phase ^= 1;
         tc_fence_after();
-#ifdef NERF_PIPE_EXP_NOEPI
-        for (int ph = 0; ph < 2; ++ph) {
-          if (ev > 0) mbar_wait(bar_img_empty, (ev - 1) & 1u);
-          if (ph == 1) {
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive_cluster(acc_free_leader);
-          }
-          __syncwarp();
-          if (lane == 0) mbar_arrive(bar_img_full);
-          ++ev;
-        }
-        continue;
-#endif
 #pragma unroll 1
         for (int ph = 0; ph < 2; ++ph) {
           const int col0 = 128 * ph + 64 * hh;                       // first accumulator column of this warp in this phase
@@ -709,11 +695,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(pipe::kThreads, 1) m
         prefetch_group(t + kPrefetchAhead);
         for (int i = 0; i < 12; ++i) {
           mbar_wait(bar_full + 8 * stage, phase);
-#ifdef NERF_PIPE_EXP_NORED
-          if (false) {
-#else
           if (i >= 4) {
-#endif
             const int q = (i - 4) >> 2, xy = ((i - 4) >> 1) & 1, j = i & 1;
             const uint32_t base = smem_base + kOffRing + stage * kStageBytes;
             if (xy == 0) {
@@ -793,11 +775,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(pipe::kThreads, 1) m
               if (lane == 0) PIPE_TIMED(s_freed, spin_until(flag_freed(st, ls), 2u * (uint32_t)use));
               __syncwarp();
             }
-#ifndef NERF_PIPE_EXP_NOSTORE
             uint4* dst = reinterpret_cast<uint4*>(link_base(st, ls) + rank * kActBytes + img_off);
 #pragma unroll
             for (int i = 0; i < 16; ++i) dst[i * 32 + lane] = v[i];
-#endif
           }
           if (gregion >= 0 && tile_ok) {
             uint4* dst = reinterpret_cast<uint4*>(p.gstash + grad_region_offset(gregion, n_tiles64) + (uint64_t)tile * kActBytes + img_off);

@@ -40,42 +40,6 @@
 #include "tc.cuh"
 #include "../../include/nerf_b200.h"
 
-#if defined(NERF_EXP_LSU_STORE) || defined(NERF_EXP_PACED_STORE)
-#define NERF_EXP_STORE_WARPS 1
-#endif
-// operands are handed to the MMA issuer per warp BEFORE the slot's warps meet for the image store / bias refill (measured in round 2:
-// inference 0.689 -> 0.667 ms at 4096 x 192, training unchanged); -DNERF_LATE_HANDOFF restores the round-1 order for A/B timing
-#if !defined(NERF_LATE_HANDOFF) && !defined(NERF_EXP_STORE_WARPS) && !defined(NERF_EXP_EARLY_HANDOFF)
-#define NERF_EXP_EARLY_HANDOFF 1
-#endif
-// -DNERF_EXP_CPASYNC_W: in training the weight ring is filled by LSU cp.async (32 lanes x 16 B) instead of bulk copies, so
-// the loads no longer queue behind 64 KB image stores in the TMA unit (DESIGN.md 4a fact 3); _ALL does it in inference too
-#if defined(NERF_EXP_CPASYNC_W_ALL)
-#define NERF_LSU_W(train) true
-#elif defined(NERF_EXP_CPASYNC_W)
-#define NERF_LSU_W(train) (train)
-#else
-#define NERF_LSU_W(train) false
-#endif
-// Shared weight stages (default since round 2; -DNERF_NO_SHARE_W restores one load per slot): the two slots of a CTA walk the
-// chain one stage apart, so the weight panels of stage st are needed by slot 0 and, one accumulator later, by slot 1. They are
-// loaded ONCE; slot 1's MMAs release the ring stages (half the L2 -> SM weight stream). Only stages whose panels all fit in the
-// ring can be shared (slot 0 holds them until slot 1 is done): every stage but the two 5-panel ones (skip layer, colour layer).
-// Measured (profiles/r02_chain_kernel_experiments.txt): the issuer's W-full wait halves and its A-ready wait grows by almost
-// as much -- the epilogue is the critical path -- so the gain is 1-2 % (inference 0.674 -> 0.667 ms, training 1.051 -> 1.038).
-#if defined(NERF_NO_SHARE_W)
-#define NERF_SHARE_W(train) false
-#else
-#define NERF_SHARE_W(train) true
-#endif
-#ifndef NERF_EXP_CPASYNC_MODE   // 0: cp.async.mbarrier.arrive.noinc + consumer-side proxy fence; 2: commit/wait groups + writer-side fence + plain arrive
-#define NERF_EXP_CPASYNC_MODE 0
-#endif
-constexpr uint32_t kLsuLag = 2;
-#ifndef NERF_EXP_PIECE
-#define NERF_EXP_PIECE 8192u
-#endif
-
 namespace nerf {
 using namespace tc;
 
@@ -83,10 +47,7 @@ namespace fwd {
 constexpr int kEpiThreadsPerSlot = 256;  // 8 warps: 4 TMEM lane quarters x 2 column halves
 constexpr int kThreads = 128 + 2 * kEpiThreadsPerSlot;
 // weight ring: 16 KB stages = one K panel (64 inputs) x this CTA's 128 output neurons (64 for the colour layer)
-#ifndef NERF_FWD_RING
-#define NERF_FWD_RING 4
-#endif
-constexpr int kRingStages = NERF_FWD_RING;
+constexpr int kRingStages = 4;
 constexpr uint32_t kRingStageBytes = kPanelBytes128;
 // shared memory map (offsets from the 1024-aligned base)
 constexpr uint32_t kSlotBytes = kActBytes + kPanelBytes128;  // act (4 panels) + enc (1 panel)
@@ -152,19 +113,20 @@ __device__ __forceinline__ void write_half_row(uint32_t panel_smem, int row, int
 
 // Half (16 columns, kOff = 0 or 16) of a 32-column chunk of a hidden-stage epilogue: x = acc + bias [ReLU] -> fp16
 // pairs -> two 16-byte chunks of the swizzled A operand; c0 = byte offset of the 32-column chunk in the (unswizzled)
-// panel row.  The bias comes from the slot's shared-memory copy (one broadcast LDS.128 per four columns; from global
-// memory every ~20th load missed the 28 KB L1 and stalled the warp for an L2 round trip).  Returns the ReLU bits of
-// these 16 columns (tc.cuh relu_mask_bit layout); accumulates the density head (fp32, weights at ws) when kDens.
+// panel row.  breg holds the bias of these 16 columns, loaded by the caller from the slot's shared-memory copy (one
+// broadcast LDS.128 per four columns; from global memory every ~20th load missed the 28 KB L1 and stalled the warp for
+// an L2 round trip).  Returns the ReLU bits of these 16 columns (tc.cuh relu_mask_bit layout); accumulates the density
+// head (fp32, weights at ws) when kDens.
 template <bool kDens, bool kMask, int kOff>
-__device__ __forceinline__ uint32_t hidden16(const uint32_t (&v)[32], const float4* __restrict__ b, const float* __restrict__ ws, bool relu,
-                                             uint32_t pbase, uint32_t c0, uint32_t xr, float& dens, const float4* breg = nullptr) {
+__device__ __forceinline__ uint32_t hidden16(const uint32_t (&v)[32], const float* __restrict__ ws, bool relu,
+                                             uint32_t pbase, uint32_t c0, uint32_t xr, float& dens, const float4* breg) {
   uint32_t m = 0;
   uint32_t w[8];
 #pragma unroll
   for (int qq = 0; qq < 4; ++qq) {
     constexpr int kQ0 = kOff / 4;
     const int q = kQ0 + qq;  // index of the 4-column group within the 32-column chunk
-    const float4 bq = breg != nullptr ? breg[qq] : b[q];   // (breg: loaded one 16-column group ahead by the caller)
+    const float4 bq = breg[qq];   // (loaded one 16-column group ahead by the caller)
     float x0 = __uint_as_float(v[4 * q + 0]) + bq.x;
     float x1 = __uint_as_float(v[4 * q + 1]) + bq.y;
     float x2 = __uint_as_float(v[4 * q + 2]) + bq.z;
@@ -223,17 +185,19 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
   const uint32_t bar_acc_ready = bar_a_ready + 16;        // [2] accumulator complete (multicast commit)
   const uint32_t bar_bias = bar_acc_ready + 16;           // [2] the slot's bias vector of the next stage has landed
   const uint32_t tmem_slot = bar_bias + 16;               // uint32: TMEM base address
-  const uint32_t bar_img_full = tmem_slot + 16;           // [2] (LSU-store experiment) the slot's stash image is complete in shared memory
-  const uint32_t bar_img_empty = bar_img_full + 16;       // [2] ... and has been copied out by the slot's store warp
   const uint32_t rank = cluster_ctarank();                // 0 = leader
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  constexpr bool kLsuW = NERF_LSU_W(kTrain);
-  constexpr bool kShareW = NERF_SHARE_W(kTrain);
-  auto shared_stage = [&](int st) { return kShareW && fwd_panels(st) <= kRingStages; };
+  // Shared weight stages: the two slots of a CTA walk the chain one stage apart, so the weight panels of stage st are needed
+  // by slot 0 and, one accumulator later, by slot 1. They are loaded ONCE; slot 1's MMAs release the ring stages (half the
+  // L2 -> SM weight stream). Only stages whose panels all fit in the ring can be shared (slot 0 holds them until slot 1 is
+  // done): every stage but the two 5-panel ones (skip layer, colour layer).
+  // Measured (profiles/r02_chain_kernel_experiments.txt): the issuer's W-full wait halves and its A-ready wait grows by almost
+  // as much -- the epilogue is the critical path -- so the gain is 1-2 % (inference 0.674 -> 0.667 ms, training 1.051 -> 1.038).
+  auto shared_stage = [&](int st) { return fwd_panels(st) <= kRingStages; };
   if (threadIdx.x == 0) {
     for (int i = 0; i < kRingStages; ++i) {
-      mbar_init(bar_w_full + 8 * i, (kLsuW && NERF_EXP_CPASYNC_MODE != 2) ? 32 : 1);   // LSU ring: one cp.async-completion arrival per producer lane
+      mbar_init(bar_w_full + 8 * i, 1);
       mbar_init(bar_w_empty + 8 * i, 1);
       mbar_init(bar_w_peer + 8 * i, 1);
     }
@@ -241,8 +205,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
       mbar_init(bar_a_ready + 8 * s, 16);  // one arrival per epilogue warp of either CTA
       mbar_init(bar_acc_ready + 8 * s, 1);
       mbar_init(bar_bias + 8 * s, 1);
-      mbar_init(bar_img_full + 8 * s, 8);   // one arrival per epilogue warp of the slot
-      mbar_init(bar_img_empty + 8 * s, 1);
     }
     fence_barrier_init();
   }
@@ -271,9 +233,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
       // one ring stage per K panel: rows [128 * rank, +128) of the 256-neuron panels, [64 * rank, +64) of the
       // 128-neuron colour-layer panels (the cta_group::2 MMA takes the other half from the peer's ring)
       uint32_t stage = 0, phase = 0;
-      uint32_t lsu_issued = 0, lsu_sig = 0;   // (cp.async ring, mode 2) stages issued / next stage to announce
-      (void)lsu_issued;
-      (void)lsu_sig;
       const uint64_t keep = l2_evict_last();
       long long t_wait = 0;
       const long long t_begin = prof_on ? clock64() : 0;
@@ -286,25 +245,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
             const uint32_t bytes = st == 9 ? kRingStageBytes / 2 : kRingStageBytes;  // colour layer: 64 of 128 neurons
             for (int pp = 0; pp < np; ++pp) {
               NERF_TIMED(prof_on, t_wait, mbar_wait(bar_w_empty + 8 * stage, phase ^ 1));
-              if (kLsuW) {
-                const uint8_t* src = p.packed + fwd_panel_offset(first + pp) + rank * bytes + lane * 16;
-                const uint32_t dst = smem_base + kOffRing + stage * kRingStageBytes + lane * 16;
-#pragma unroll 8
-                for (uint32_t off = 0; off < bytes; off += 512) cp_async16(dst + off, src + off);
-#if NERF_EXP_CPASYNC_MODE == 2
-                // writer-side completion: the stage issued kLsuLag stages ago has landed -> fence to the async proxy -> one arrival
-                cp_async_commit();
-                if (++lsu_issued > kLsuLag) {
-                  cp_async_wait<kLsuLag>();
-                  fence_proxy_async_smem();
-                  __syncwarp();
-                  if (lane == 0) mbar_arrive(bar_w_full + 8 * lsu_sig);
-                  if (++lsu_sig == kRingStages) lsu_sig = 0;
-                }
-#else
-                cp_async_mbar_arrive_noinc(bar_w_full + 8 * stage);
-#endif
-              } else if (elect_one()) {
+              if (elect_one()) {
                 mbar_arrive_expect_tx(bar_w_full + 8 * stage, bytes);
                 bulk_g2s_hint(smem_base + kOffRing + stage * kRingStageBytes, p.packed + fwd_panel_offset(first + pp) + rank * bytes, bytes,
                               bar_w_full + 8 * stage, keep);
@@ -318,18 +259,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
           }
         }
       }
-#if NERF_EXP_CPASYNC_MODE == 2
-      if (kLsuW) {
-        cp_async_wait<0>();
-        fence_proxy_async_smem();
-        __syncwarp();
-        const uint32_t left = lsu_issued < kLsuLag ? lsu_issued : kLsuLag;
-        for (uint32_t i = 0; i < left; ++i) {
-          if (lane == 0) mbar_arrive(bar_w_full + 8 * lsu_sig);
-          if (++lsu_sig == kRingStages) lsu_sig = 0;
-        }
-      }
-#endif
       if (prof_on && lane == 0) {
         atomicAdd(p.prof + 3, (unsigned long long)t_wait);
         atomicAdd(p.prof + 4, (unsigned long long)(clock64() - t_begin));
@@ -364,7 +293,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
             for (int pp = 0; pp < np; ++pp) {
               NERF_TIMED(prof_on, t_w, mbar_wait(bar_w_full + 8 * stage, phase));
               NERF_TIMED(prof_on, t_w, mbar_wait_cluster(bar_w_peer + 8 * stage, phase));
-              if (kLsuW && NERF_EXP_CPASYNC_MODE != 2) fence_proxy_async_smem();   // cp.async data arrived through the generic proxy
               tc_fence_after();
               if (elect_one()) {
                 // A: stage 0 reads the encoding panel; panel 4 of stages 5 / 9 is the encoding / direction panel
@@ -393,75 +321,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
         atomicAdd(p.prof + 2, (unsigned long long)(clock64() - t_begin));
         atomicAdd(p.prof + 9, 1ull);
       }
-#if defined(NERF_EXP_STORE_WARPS)
-    } else if (warp >= 2) {
-      // =============================== stash store warps (one per slot) ===============================
-      // Measured (tools/l2_probe.py): one SM's TMA engine moves 66 B/clk of bulk loads but only 27-32 B/clk of bulk stores,
-      // and a queued 64 KB image store delays the weight-ring loads behind it (the issuer's W-full wait tripled in training).
-      // Here the images leave through the LSU instead: a linear 16-byte copy shared -> global (the stash image IS the
-      // shared-memory image), one warp per slot, so the TMA engine only carries the weight ring.
-      if (kTrain) {
-        const int slot = warp - 2;
-        const uint32_t act = smem_base + slot * kSlotBytes;
-        const uint8_t* act_g = smem_raw + slot * kSlotBytes;
-        const uint64_t n_tiles64 = (uint64_t)p.n_tiles;
-        uint32_t ph = 0;
-        (void)act;
-#if defined(NERF_EXP_LSU_STORE)
-        auto copy_out = [&](int region, const uint8_t* src, uint32_t bytes, int tile) {
-          uint4* dst = reinterpret_cast<uint4*>(p.stash + stash_region_offset(region, n_tiles64) + (uint64_t)tile * stash_region_tile_bytes(region));
-          const uint4* sp = reinterpret_cast<const uint4*>(src);
-          const int n16 = (int)(bytes >> 4);
-#pragma unroll 2
-          for (int q = lane; q < n16; q += 64) {
-            const uint4 v0 = sp[q], v1 = sp[q + 32];
-            __stcs(dst + q, v0);
-            __stcs(dst + q + 32, v1);
-          }
-        };
-#else
-        // PACED bulk stores: the image leaves in 8 KB pieces and the next piece is only issued when the previous one has been
-        // read out of shared memory, so the TMA unit's queue never holds more than one store piece of this slot and a weight-ring
-        // load queued by the producer warp waits for ~300 cycles of store instead of a whole 64 KB image (~2,200 cycles at the
-        // SM's 27-32 B/clk store path; measured: the issuer's W-full wait tripled in training).
-        const uint64_t pol = l2_evict_first();
-        auto copy_out = [&](int region, const uint8_t* src, uint32_t bytes, int tile) {
-          uint8_t* dst = p.stash + stash_region_offset(region, n_tiles64) + (uint64_t)tile * stash_region_tile_bytes(region);
-          const uint32_t s_addr = smem_base + (uint32_t)(src - smem_raw);
-          if (lane == 0) {
-            for (uint32_t off = 0; off < bytes; off += NERF_EXP_PIECE) {
-              bulk_s2g_hint(dst + off, s_addr + off, NERF_EXP_PIECE, pol);
-              bulk_commit();
-              bulk_wait_read<0>();
-            }
-          }
-          __syncwarp();
-        };
-#endif
-        for (int it = 0; it < n_iters; ++it) {
-          if (!active(it, slot)) break;
-          const int tile = group_of(it, slot) * 2 + (int)rank;
-          const bool tile_ok = tile < p.n_tiles;
-          for (int ev = 0; ev < 11; ++ev) {   // ENC | H0..H7 | DIR + F | G  (the epilogue's event sequence)
-            mbar_wait(bar_img_full + 8 * slot, ph);
-            if (tile_ok) {
-              if (ev == 0) copy_out(kStashEnc, act_g + kActBytes, kPanelBytes128, tile);
-              else if (ev <= 8) copy_out(kStashH0 + ev - 1, act_g, kActBytes, tile);
-              else if (ev == 9) {
-                copy_out(kStashDir, act_g + kActBytes, kPanelBytes128, tile);
-                copy_out(kStashF, act_g, kActBytes, tile);
-              } else copy_out(kStashG, act_g, 2 * kPanelBytes128, tile);
-            }
-            __syncwarp();
-            if (lane == 0) mbar_arrive(bar_img_empty + 8 * slot);
-            ph ^= 1;
-          }
-        }
-      }
     } else if (warp == 1) {
-#else
-    } else if (warp == 1) {
-#endif
       // =============================== relay (peer CTA) ===============================
       // tells the leader's issuer that this CTA's half of ring stage s has landed (bulk copies can only signal a
       // barrier of their own CTA, and mbarriers cannot be waited on remotely)
@@ -474,7 +334,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
             const int np = fwd_panels(st);
             for (int pp = 0; pp < np; ++pp) {
               mbar_wait(bar_w_full + 8 * stage, phase);
-              if (kLsuW && NERF_EXP_CPASYNC_MODE != 2) fence_proxy_async_smem();   // this CTA's half: fenced here, the leader's issuer only sees the relay
               if (elect_one()) mbar_arrive_cluster(mapa(bar_w_peer + 8 * stage, 0));
               __syncwarp();
               if (++stage == kRingStages) {
@@ -505,9 +364,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
     const uint32_t t_acc = t_slot + 128 * half;                            // hidden stages: columns [128 * half, +128)
     const uint32_t act_h = act + 2 * half * kPanelBytes128 + row_off;      // this row in the first of this half's two panels
     uint32_t acc_phase = 0, bias_phase = 0;
-    uint32_t img_events = 0, img_drained = 0;   // (LSU-store experiment) stash images handed to / finished by the slot's store warp
-    (void)img_events;
-    (void)img_drained;
     const uint64_t n_tiles64 = (uint64_t)p.n_tiles;
     const uint32_t a_ready_leader = mapa(bar_a_ready + 8 * slot, 0);  // both CTAs announce their operands to the leader
     const bool prof = prof_on && tg == 0 && slot == 0;
@@ -538,34 +394,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
       // stash helper: one thread bulk-stores an image from shared memory after the slot's warps fenced their writes
       auto stash_issue = [&](int region, uint32_t src, uint32_t bytes) {  // one thread, after the slot's warps fenced + met
         if (tg == 0 && tile_ok) {
-          #if defined(NERF_EXP_STORE_WRAP)   // diagnostic: every image lands in a 16-tile window that stays in L2 (results are wrong downstream)
-          const uint64_t tile_w = (uint64_t)(tile & 15);
-#else
-          const uint64_t tile_w = (uint64_t)tile;
-#endif
-          uint8_t* dst = p.stash + stash_region_offset(region, n_tiles64) + tile_w * stash_region_tile_bytes(region);
-#if defined(NERF_EXP_NOSTORE)
-          (void)dst;
-#elif defined(NERF_EXP_SPLIT_STORE)
-          for (uint32_t off = 0; off < bytes; off += kPanelBytes128) bulk_s2g_hint(dst + off, src + off, kPanelBytes128, l2_evict_first());
-#elif defined(NERF_EXP_NOHINT)
-          bulk_s2g(dst, src, bytes);
-#else
+          uint8_t* dst = p.stash + stash_region_offset(region, n_tiles64) + (uint64_t)tile * stash_region_tile_bytes(region);
           bulk_s2g_hint(dst, src, bytes, l2_evict_first());
-#endif
           bulk_commit();
         }
       };
-#if defined(NERF_EXP_STORE_WARPS)
-      auto stash_store = [&](int region, uint32_t src, uint32_t bytes) {   // event: this warp's part of the image is in shared memory
-        if (kTrain && region != kStashDir) {                                 // (DIR leaves together with F: one event)
-          fence_proxy_async_smem();                                          // (bulk stores read the image through the async proxy)
-          __syncwarp();
-          if (lane == 0) mbar_arrive(bar_img_full + 8 * slot);
-          ++img_events;
-        }
-      };
-#else
       auto stash_store = [&](int region, uint32_t src, uint32_t bytes) {
         if (kTrain) {
           fence_proxy_async_smem();
@@ -573,18 +406,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
           stash_issue(region, src, bytes);
         }
       };
-#endif
       // before overwriting a buffer that may still be read by an in-flight bulk store
-#if defined(NERF_EXP_STORE_WARPS)
-      auto stash_drain = [&]() {   // every event issued so far has been copied out (at most one is outstanding)
-        if (kTrain && img_events != img_drained) {
-          const long long t0 = prof ? clock64() : 0;
-          mbar_wait(bar_img_empty + 8 * slot, (img_events - 1) & 1u);
-          img_drained = img_events;
-          if (prof) t_drain += clock64() - t0;
-        }
-      };
-#else
       auto stash_drain = [&]() {
         if (kTrain) {
           const long long t0 = prof ? clock64() : 0;
@@ -593,7 +415,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
           if (prof) t_drain += clock64() - t0;
         }
       };
-#endif
 
       // ---------------- prologue: position encoding -> enc panel (each half writes its 32 of the 64 columns) ----------------
       // columns: [x y z | enc(x) 3..22 | enc(y) 23..42 | enc(z) 43..62 | 0]; half 0 needs enc(x) and the first nine
@@ -679,11 +500,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
           tmem_ld32(t_acc, va);
           stash_drain();  // the act image of the previous stage may still be being stored
           NERF_TIMED(prof, t_bias, mbar_wait(bar_bias + 8 * slot, bias_phase));
-#if !defined(NERF_NO_BIAS_AHEAD)
           // The bias words of 16-column group g + 1 are loaded BEFORE the (asm volatile, "memory") stores of group g: the compiler
           // cannot move the LDS across them by itself, and ncu's source view showed the first FADD of every group waiting on it
           // (13 % of the epilogue warps' samples).  Measured (round 2, profiles/r02_chain_kernel_experiments.txt): training
-          // forward 1.049 -> 0.972 ms, inference 0.703 -> 0.695 ms; -DNERF_NO_BIAS_AHEAD restores the in-place loads.
+          // forward 1.049 -> 0.972 ms, inference 0.703 -> 0.695 ms.
           float4 ba[4], bb[4];
           auto load4 = [&](float4 (&dst)[4], int group) {   // group = 16-column group index within this thread's 128 columns
 #pragma unroll
@@ -695,33 +515,19 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
             const uint32_t pbase = act_h + (uint32_t)(c >> 1) * kPanelBytes128;
             tmem_ld_wait32(va);
             load4(bb, 2 * c + 1);
-            mw[c] = hidden16<kDens, kTrain, 0>(va, bsp, wsp + 32 * c, relu, pbase, 0u, xr, dens, ba);
+            mw[c] = hidden16<kDens, kTrain, 0>(va, wsp + 32 * c, relu, pbase, 0u, xr, dens, ba);
             tmem_ld32(t_acc + 32 * (c + 1), vb);
             load4(ba, 2 * c + 2);
-            mw[c] |= hidden16<kDens, kTrain, 16>(va, bsp, wsp + 32 * c, relu, pbase, 0u, xr, dens, bb);
+            mw[c] |= hidden16<kDens, kTrain, 16>(va, wsp + 32 * c, relu, pbase, 0u, xr, dens, bb);
             tmem_ld_wait32(vb);
             load4(bb, 2 * c + 3);
-            mw[c + 1] = hidden16<kDens, kTrain, 0>(vb, bsp, wsp + 32 * (c + 1), relu, pbase, 64u, xr, dens, ba);
+            mw[c + 1] = hidden16<kDens, kTrain, 0>(vb, wsp + 32 * (c + 1), relu, pbase, 64u, xr, dens, ba);
             if (c + 2 < 4) {
               tmem_ld32(t_acc + 32 * (c + 2), va);
               load4(ba, 2 * c + 4);
             }
-            mw[c + 1] |= hidden16<kDens, kTrain, 16>(vb, bsp, wsp + 32 * (c + 1), relu, pbase, 64u, xr, dens, bb);
+            mw[c + 1] |= hidden16<kDens, kTrain, 16>(vb, wsp + 32 * (c + 1), relu, pbase, 64u, xr, dens, bb);
           }
-#else
-#pragma unroll
-          for (int c = 0; c < 4; c += 2) {
-            const uint32_t pbase = act_h + (uint32_t)(c >> 1) * kPanelBytes128;
-            tmem_ld_wait32(va);
-            mw[c] = hidden16<kDens, kTrain, 0>(va, bsp + 8 * c, wsp + 32 * c, relu, pbase, 0u, xr, dens);
-            tmem_ld32(t_acc + 32 * (c + 1), vb);
-            mw[c] |= hidden16<kDens, kTrain, 16>(va, bsp + 8 * c, wsp + 32 * c, relu, pbase, 0u, xr, dens);
-            tmem_ld_wait32(vb);
-            mw[c + 1] = hidden16<kDens, kTrain, 0>(vb, bsp + 8 * (c + 1), wsp + 32 * (c + 1), relu, pbase, 64u, xr, dens);
-            if (c + 2 < 4) tmem_ld32(t_acc + 32 * (c + 2), va);
-            mw[c + 1] |= hidden16<kDens, kTrain, 16>(vb, bsp + 8 * (c + 1), wsp + 32 * (c + 1), relu, pbase, 64u, xr, dens);
-          }
-#endif
         };
         if (st == 7) run(BoolTag<true>{}); else run(BoolTag<false>{});
         bias_phase ^= 1;
@@ -741,8 +547,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
           write_half_row(enc, row, half, vals);
           stash_store(kStashDir, enc, kPanelBytes128);
         }
-#if defined(NERF_EXP_EARLY_HANDOFF)
         // operands are handed to the MMA issuer per warp BEFORE the slot's warps meet for the image store / bias refill
+        // (measured in round 2: inference 0.689 -> 0.667 ms at 4096 x 192, training unchanged)
         fence_proxy_async_smem();
         tc_fence_before();
         __syncwarp();
@@ -750,19 +556,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
         NERF_TIMED(prof, t_bar, named_bar_sync(bar_id, kEpiThreadsPerSlot));
         if (kTrain) stash_issue(st < 8 ? kStashH0 + st : kStashF, act, kActBytes);
         if (tg == 0) bias_fetch(st + 1);
-#else
-        stash_store(st < 8 ? kStashH0 + st : kStashF, act, kActBytes);  // (training) fence + slot barrier + bulk store
-        fence_proxy_async_smem();
-#if defined(NERF_EXP_STORE_WARPS)
-        named_bar_sync(bar_id, kEpiThreadsPerSlot);               // (the event hand-off above has no slot barrier of its own)
-#else
-        if (!kTrain) named_bar_sync(bar_id, kEpiThreadsPerSlot);  // every warp of the slot is done with this stage's bias
-#endif
-        if (tg == 0) bias_fetch(st + 1);
-        tc_fence_before();
-        __syncwarp();  // one (possibly remote) arrival per warp
-        if (lane == 0) mbar_arrive_cluster(a_ready_leader);
-#endif
         // ReLU bits -> stash, after the hand-off: a plain global store can stall its warp under the stash's HBM write load
         if (kTrain && relu && tile_ok) {
           uint4* md = reinterpret_cast<uint4*>(p.stash + stash_region_offset(kStashMask, n_tiles64) +
@@ -825,9 +618,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
         const uint32_t xch = act + 3 * kPanelBytes128 + (uint32_t)row * 16u;
         if (half == 1) st_shared_v4(xch, __float_as_uint(a0), __float_as_uint(a1), __float_as_uint(a2), __float_as_uint(dens));
         stash_store(kStashG, act, 2 * kPanelBytes128);  // (training) its barrier also orders the exchange
-#if defined(NERF_EXP_STORE_WARPS)
-        if (kTrain) named_bar_sync(bar_id, kEpiThreadsPerSlot);
-#endif
         if (!kTrain) {
           fence_proxy_async_smem();
           named_bar_sync(bar_id, kEpiThreadsPerSlot);
@@ -920,11 +710,7 @@ extern "C" int nerf_mlp_forward(float* rgbsigma, void* stash, const void* packed
     attr_set = true;
   }
   const cudaStream_t st = static_cast<cudaStream_t>(stream);
-#if defined(NERF_RUNTIME_PROF)   // A/B: always the instantiation that carries the counters behind a run-time flag (the round-1 build)
-  const bool with_prof = true;
-#else
   const bool with_prof = p.prof != nullptr;
-#endif
   if (stash != nullptr) {
     if (with_prof) mlp_fwd_kernel<true, true><<<grid, fwd::kThreads, fwd::kSmemBytes, st>>>(p);
     else mlp_fwd_kernel<true, false><<<grid, fwd::kThreads, fwd::kSmemBytes, st>>>(p);

@@ -201,155 +201,18 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32) importance_kernel_smem(
   for (int j = lane; j < s; j += 32) z_merged[(int64_t)ray * s + j] = merged[j];
 }
 
-// ---- K2, register flavour (n_fine <= 512) ------------------------------------------------------------
-// Same algorithm, but the Nf fine depths are sorted in REGISTERS (K = ceil(Nf/32) keys per lane, element
-// e = r * 32 + lane): compare-exchange distances below 32 are one SHFL + one predicated FMNMX per key, larger
-// distances are in-lane min/max pairs with compile-time direction; the whole network is straight-line code
-// (Nf = 128: ~260 instructions instead of ~1,400 for the shared-memory network).  The K cdf inversions of a lane
-// are independent (instruction-level parallelism hides the shared-memory latency of the binary searches), and the
-// sequential cdf sums of the block's 8 rays run side by side on 8 lanes of one warp instead of on lane 0 of
-// every warp.
-template <int K>
-__device__ __forceinline__ void bitonic_sort_regs(float (&x)[K], int lane) {
-  constexpr int N = 32 * K;
-#pragma unroll
-  for (int k = 2; k <= N; k <<= 1) {
-#pragma unroll
-    for (int j = k >> 1; j >= 1; j >>= 1) {
-      if (j < 32) {
-        const bool lower = (lane & j) == 0;
-#pragma unroll
-        for (int r = 0; r < K; ++r) {
-          const bool up = k < 32 ? ((lane & k) == 0) : (((r * 32) & k) == 0);
-          const float other = __shfl_xor_sync(0xffffffffu, x[r], j);
-          x[r] = (lower == up) ? fminf(x[r], other) : fmaxf(x[r], other);
-        }
-      } else {
-        const int jr = j >> 5;
-#pragma unroll
-        for (int r = 0; r < K; ++r) {
-          if ((r & jr) == 0) {
-            const int r2 = r | jr;
-            const bool up = ((r * 32) & k) == 0;
-            const float lo = fminf(x[r], x[r2]), hi = fmaxf(x[r], x[r2]);
-            x[r] = up ? lo : hi;
-            x[r2] = up ? hi : lo;
-          }
-        }
-      }
-    }
-  }
-}
-
-template <int K>
-__global__ void __launch_bounds__(kWarpsPerBlock * 32) importance_kernel_reg(
-    float* __restrict__ z_merged, float* __restrict__ z_fine_out, const float* __restrict__ z_coarse,
-    const float* __restrict__ w_coarse, const float* __restrict__ u, int n_rays, int nc, int nf) {
-  extern __shared__ float sm[];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int ray = blockIdx.x * kWarpsPerBlock + warp;
-  const bool active = ray < n_rays;
-  const int nb = nc - 1, nv = nc - 2, s = nc + nf;
-  const int per_warp = 3 * nb + nc + 32 * K + s;
-  float* cdf = sm + warp * per_warp;
-  float* edges = cdf + nb;
-  float* pdf = edges + nb;
-  float* zcs = pdf + nb;
-  float* fine = zcs + nc;
-  float* merged = fine + 32 * K;
-
-  if (active) {
-    const float* zc = z_coarse + (int64_t)ray * nc;
-    const float* wc = w_coarse + (int64_t)ray * nc;
-    float part = 0.f;
-    for (int j = lane; j < nc; j += 32) {
-      const float zj = __ldg(zc + j);
-      zcs[j] = zj;
-      if (j < nb) edges[j] = __fmul_rn(0.5f, __fadd_rn(zj, __ldg(zc + j + 1)));
-      if (j < nv) {
-        const float v = __fadd_rn(__ldg(wc + j + 1), 1e-5f);
-        pdf[j] = v;
-        part += v;
-      }
-    }
-    const float total = warp_sum(part);
-    for (int j = lane; j < nv; j += 32) pdf[j] = __fdiv_rn(pdf[j], total);
-  }
-  __syncthreads();
-  if (warp == 0 && lane < kWarpsPerBlock && blockIdx.x * kWarpsPerBlock + lane < n_rays) {
-    // sequential running sums (the reference's order) of the block's rays, one lane per ray
-    float* c = sm + lane * per_warp;
-    const float* pd = c + 2 * nb;
-    float run = 0.f;
-    c[0] = 0.f;
-    for (int j = 0; j < nv; ++j) {
-      run = __fadd_rn(run, pd[j]);
-      c[j + 1] = run;
-    }
-  }
-  __syncthreads();
-  if (!active) return;
-
-  float x[K];
-  const float inv_nf1 = nf > 1 ? 1.f / (float)(nf - 1) : 0.f;
-#pragma unroll
-  for (int r = 0; r < K; ++r) {
-    const int e = r * 32 + lane;
-    float uj = 0.f;
-    if (e < nf) {
-      if (u != nullptr) uj = __ldg(u + (int64_t)ray * nf + e);
-      else uj = (e < nf / 2) ? __fmul_rn(inv_nf1, (float)e) : __fsub_rn(1.f, __fmul_rn(inv_nf1, (float)(nf - e - 1)));
-    }
-    x[r] = uj;
-  }
-#pragma unroll
-  for (int r = 0; r < K; ++r) {
-    const int e = r * 32 + lane;
-    const float zf = invert_cdf(cdf, edges, nb, x[r]);
-    if (e < nf && z_fine_out != nullptr) z_fine_out[(int64_t)ray * nf + e] = zf;
-    x[r] = e < nf ? zf : __int_as_float(0x7f800000);  // +inf padding sorts to the end
-  }
-  bitonic_sort_regs<K>(x, lane);
-#pragma unroll
-  for (int r = 0; r < K; ++r) fine[r * 32 + lane] = x[r];
-  // merge by rank: position(fine e) = e + #{coarse <= z_f[e]}, position(coarse i) = i + #{fine < z_c[i]}
-  // (measured: early-exit searches beat branch-free fixed-trip ones here -- the kernel is bound by shared-memory
-  // bank conflicts of the data-dependent probes, not by issue slots, and early exit saves probes)
-#pragma unroll
-  for (int r = 0; r < K; ++r) {
-    const int e = r * 32 + lane;
-    int a = 0, b = nc;
-    while (a < b) {
-      const int mid = (a + b) >> 1;
-      if (zcs[mid] <= x[r]) a = mid + 1; else b = mid;
-    }
-    if (e < nf) merged[e + a] = x[r];
-  }
-  __syncwarp();
-  for (int i = lane; i < nc; i += 32) {
-    const float zi = zcs[i];
-    int a = 0, b = nf;
-    while (a < b) {
-      const int mid = (a + b) >> 1;
-      if (fine[mid] < zi) a = mid + 1; else b = mid;
-    }
-    merged[i + a] = zi;
-  }
-  __syncwarp();
-  for (int j = lane; j < s; j += 32) z_merged[(int64_t)ray * s + j] = merged[j];
-}
-
-
 // ---- K2, sorted-noise flavour (n_fine <= 512): the production kernel -----------------------------------
 // The inverse cdf is a composition of monotone, correctly rounded operations, so SORTING THE NOISE FIRST gives
-// the fine depths already in ascending order.  That removes three of the four costs of the flavour above:
+// the fine depths already in ascending order.  Compared with sorting the depths after the inversion (the
+// shared-memory kernel above, kept for n_fine > 512):
 //   * one binary search per LANE (for its first key) followed by monotone advances through the cdf, instead
 //     of one binary search per SAMPLE;
 //   * no search at all to place fine samples among the coarse ones, and none to place coarse among fine: the two
 //     ascending lists are merged by MERGE PATH (every lane binary-searches its diagonal once and then emits
 //     ceil(S/32) consecutive outputs sequentially);
-//   * the register sort uses a BLOCKED layout (lane owns K consecutive keys, loaded as float4): compare-exchange
-//     distances below K stay inside the lane, so 15 of the 28 stages of a 128-key network need no shuffle.
+//   * the noise is sorted in registers in a BLOCKED layout (lane owns K consecutive keys, loaded as float4):
+//     compare-exchange distances below K stay inside the lane, so 15 of the 28 stages of a 128-key network need
+//     no shuffle.
 // Exactness: the fine depths are checked for sortedness (one shuffle) and re-sorted by the same network in the
 // (never observed) case of a violation, so the output is bit-identical to sort(cat(z_c, z_f)).  The sequential cdf
 // (the reference's summation order) is kept.
@@ -602,11 +465,7 @@ extern "C" int nerf_sample_importance(float* z_merged, float* z_fine, const floa
   const int blocks = (n_rays + kWarpsPerBlock - 1) / kWarpsPerBlock;
   int cdf_pad = 8;   // power of two >= number of cdf entries (n_coarse - 1): the branch-free search probes a padded table
   while (cdf_pad < n_coarse) cdf_pad <<= 1;         // the search covers cdf_pad - 1 entries
-#ifdef NERF_K2_LEGACY
-  const size_t smem = sizeof(float) * kWarpsPerBlock * (3 * (n_coarse - 1) + n_coarse + nf_pad + n_coarse + n_fine);
-#else
   const size_t smem = sizeof(float) * kWarpsPerBlock * (cdf_pad + 2 * (n_coarse - 1) + (n_coarse + 1) + (nf_pad + 1) + n_coarse + n_fine);
-#endif
   cudaStream_t st = static_cast<cudaStream_t>(stream);
 #define NERF_LAUNCH_K2_FN(FN)                                                                                                \
   do {                                                                                                                       \
@@ -616,9 +475,6 @@ extern "C" int nerf_sample_importance(float* z_merged, float* z_fine, const floa
     }                                                                                                                        \
     FN<<<blocks, kWarpsPerBlock * 32, smem, st>>>(z_merged, z_fine, z_coarse, w_coarse, u, n_rays, n_coarse, n_fine);       \
   } while (0)
-#ifdef NERF_K2_LEGACY
-#define NERF_LAUNCH_K2(KK) NERF_LAUNCH_K2_FN(importance_kernel_reg<KK>)
-#else
 #define NERF_LAUNCH_K2(KK)                                                          \
   do {                                                                              \
     switch (cdf_pad) {                                                              \
@@ -631,7 +487,6 @@ extern "C" int nerf_sample_importance(float* z_merged, float* z_fine, const floa
       default: NERF_LAUNCH_K2_FN((importance_kernel_sorted<KK, 512>)); break;       \
     }                                                                               \
   } while (0)
-#endif
   switch (nf_pad / 32) {
     case 1: NERF_LAUNCH_K2(1); break;
     case 2: NERF_LAUNCH_K2(2); break;

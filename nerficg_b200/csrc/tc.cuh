@@ -93,24 +93,6 @@ __device__ __forceinline__ void bulk_s2g_hint(void* dst, uint32_t src_smem, uint
                "l"(policy)
                : "memory");
 }
-// ---- LSU async copies (non-bulk cp.async): a second global -> shared path that does not queue behind bulk stores in the
-// SM's TMA unit. The data arrives through the generic proxy: consumers that read it through the async proxy (UMMA operand
-// reads) need fence.proxy.async after they have observed the barrier.
-// (no L2 cache-hint flavour: `cp.async.cg...L2::cache_hint` with a createpolicy evict_last policy assembles for sm_100a but
-// the resulting LDGSTS raises "illegal instruction" on B200 -- compute-sanitizer, round 2)
-__device__ __forceinline__ void cp_async16(uint32_t dst_smem, const void* src) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst_smem), "l"(src) : "memory");
-}
-// the barrier receives one arrival from this thread when all of its earlier cp.async have landed (the barrier's expected
-// count must already include it: .noinc)
-__device__ __forceinline__ void cp_async_mbar_arrive_noinc(uint32_t bar) {
-  asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() {   // all but this thread's newest N groups have landed
-  asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
-}
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 // all but the newest N bulk stores have finished READING shared memory
 template <int N>

@@ -3,7 +3,7 @@
 # usage: bash tools/gpu_session.sh <tag> [steps...]   steps: tests variants stress bench ncu
 set -u
 TAG=$1; shift
-STEPS=${*:-tests variants stress bench}
+STEPS=${*:-tests stress bench}
 OUT=gpurun_out/$TAG
 mkdir -p $OUT
 nvidia-smi --query-gpu=name,power.limit,clocks.max.sm --format=csv > $OUT/gpu.txt 2>&1
@@ -14,7 +14,7 @@ for s in $STEPS; do
       cp gpurun_out/parity_measured.jsonl $OUT/ 2>/dev/null; cp gpurun_out/grad_parity.jsonl $OUT/ 2>/dev/null;;
     variants)
       timeout 300 python tools/kernel_timing.py > $OUT/stall_base.txt 2>&1
-      for v in ${VARIANTS:-nostore early split nohint earlysplit}; do
+      for v in ${VARIANTS}; do
         NERF_B200_LIB=nerficg_b200/libnerf_b200.$v.so timeout 150 python tools/kernel_timing.py > $OUT/stall_$v.txt 2>&1
       done;;
     vtests)   # parity tests of the MLP / renderer / trained-regime suites against a variant build

@@ -10,26 +10,7 @@ sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
 from nerficg_b200.csrc import build as B  # noqa: E402
 
 VARIANTS = {
-    'nostore': ('NERF_EXP_NOSTORE',),            # diagnostic: chain kernels without their image stores (results are wrong downstream)
-    'early': ('NERF_EXP_EARLY_HANDOFF',),        # operand hand-off before the slot barrier of the image store
-    'split': ('NERF_EXP_SPLIT_STORE',),          # 4 x 16 KB stores instead of one 64 KB store
-    'nohint': ('NERF_EXP_NOHINT',),              # stores without the L2 evict_first policy
-    'earlysplit': ('NERF_EXP_EARLY_HANDOFF', 'NERF_EXP_SPLIT_STORE'),
-    'lsu': ('NERF_EXP_LSU_STORE',),              # forward stash images leave through LSU store warps instead of TMA bulk stores
-    'pipe_nored': ('NERF_PIPE_EXP_NORED',),      # fused-backward diagnostics: reducers / epilogue arithmetic / link stores switched off
-    'pipe_noepi': ('NERF_PIPE_EXP_NOEPI',),
-    'pipe_nostore': ('NERF_PIPE_EXP_NOSTORE',),
-    'pipe_none': ('NERF_PIPE_EXP_NORED', 'NERF_PIPE_EXP_NOEPI', 'NERF_PIPE_EXP_NOSTORE'),
-    'paced8': ('NERF_EXP_PACED_STORE',),         # forward stash images leave as paced 8 KB bulk stores issued by one store warp per slot
-    'paced16': ('NERF_EXP_PACED_STORE', 'NERF_EXP_PIECE=16384u'),
-    'paced4': ('NERF_EXP_PACED_STORE', 'NERF_EXP_PIECE=4096u'),
-    'lsuw': ('NERF_EXP_CPASYNC_W',),             # weight rings of the training forward and dgrad filled by LSU cp.async instead of bulk copies
-    'lsuw2': ('NERF_EXP_CPASYNC_W', 'NERF_EXP_CPASYNC_MODE=2'),   # ... commit/wait groups, writer-side proxy fence, plain arrive
-    'lsuw_all': ('NERF_EXP_CPASYNC_W_ALL',),     # ... and of the inference forward
-    'nosharew': ('NERF_NO_SHARE_W',),            # one weight load per slot and stage (the round-1 producer)
-    'nobiasahead': ('NERF_NO_BIAS_AHEAD',),      # forward: bias words loaded in place (before round 2's one-group-ahead prefetch)
-    'runtimeprof': ('NERF_RUNTIME_PROF',),       # forward: always the instantiation with the stall counters behind a run-time flag
-    'wrap': ('NERF_EXP_STORE_WRAP',),            # diagnostic: image stores hit a 16-tile window that stays in L2 (no HBM writes)
+    'pipe': ('NERF_BWD_PIPE',),                  # nerf_mlp_backward runs the fused layer-stationary backward (mlp_bwd_pipe.cu)
 }
 
 if __name__ == '__main__':
