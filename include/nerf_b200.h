@@ -104,16 +104,7 @@ int nerf_mlp_backward(float* grads, const float* d_rgbsigma, const float* rgbsig
                       const void* packed, const float* params, int n_rays, int n_samples, float grad_scale,
                       void* stream);
 
-/* nerf_mlp_backward runs the fused, layer-stationary pipeline (csrc/mlp_bwd_pipe.cu: data and weight gradients in one kernel, the
- * per-layer output gradients never leave the chip) followed by a small residual weight-gradient kernel.  The same entry point is
- * exported under its own name, and the previous two-kernel path (tile-major dgrad chain + layer-major wgrad) as *_legacy. */
-int nerf_mlp_backward_pipe(float* grads, const float* d_rgbsigma, const float* rgbsigma, const void* stash, void* workspace,
-                           const void* packed, const float* params, int n_rays, int n_samples, float grad_scale, void* stream);
-int nerf_mlp_backward_legacy(float* grads, const float* d_rgbsigma, const float* rgbsigma, const void* stash, void* workspace,
-                             const void* packed, const float* params, int n_rays, int n_samples, float grad_scale, void* stream);
-size_t nerf_mlp_backward_pipe_workspace_bytes(void);
-
-/* The two phases of the legacy path, separately launchable (profiling):
+/* The two phases of nerf_mlp_backward, separately launchable (profiling):
  * dgrad walks the chain backwards per tile and fills `workspace` with the per-layer output gradients;
  * wgrad reduces activations x gradients over all samples into `grads` (layer-major, HBM-bound). */
 int nerf_mlp_backward_dgrad(const float* d_rgbsigma, const float* rgbsigma, const void* stash, void* workspace,

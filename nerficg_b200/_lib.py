@@ -29,9 +29,6 @@ _PROTOTYPES = {
     'nerf_mlp_forward': (c_int, [c_void_p] * 9 + [c_int, c_int, c_void_p]),
     'nerf_mlp_backward_workspace_bytes': (c_size_t, [c_int64]),
     'nerf_mlp_backward': (c_int, [c_void_p] * 7 + [c_int, c_int, c_float, c_void_p]),
-    'nerf_mlp_backward_pipe': (c_int, [c_void_p] * 7 + [c_int, c_int, c_float, c_void_p]),
-    'nerf_mlp_backward_legacy': (c_int, [c_void_p] * 7 + [c_int, c_int, c_float, c_void_p]),
-    'nerf_mlp_backward_pipe_workspace_bytes': (c_size_t, []),
     'nerf_mlp_backward_dgrad': (c_int, [c_void_p] * 6 + [c_int, c_int, c_void_p]),
     'nerf_mlp_backward_wgrad': (c_int, [c_void_p] * 3 + [c_int, c_int, c_float, c_void_p]),
     'nerf_adam_tick': (c_int, [c_void_p, c_float, c_float, c_void_p]),

@@ -22,11 +22,7 @@ FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std
          '--expt-relaxed-constexpr', '-Xptxas', '-v']
 
 
-def build(force: bool = False, verbose: bool = False, defines: tuple[str, ...] = (), tag: str = '') -> Path:
-    """`defines`/`tag`: development variants (tools/variants.py): objects in build/<tag>/, library libnerf_b200.<tag>.so."""
-    global BUILD, LIB
-    if tag:
-        BUILD, LIB, force = CSRC / 'build' / tag, PKG / f'libnerf_b200.{tag}.so', True
+def build(force: bool = False, verbose: bool = False) -> Path:
     BUILD.mkdir(exist_ok=True, parents=True)
     sources = sorted(CSRC.glob('*.cu'))
     headers = list(CSRC.glob('*.cuh')) + [PKG.parent / 'include' / 'nerf_b200.h']
@@ -36,7 +32,7 @@ def build(force: bool = False, verbose: bool = False, defines: tuple[str, ...] =
         obj = BUILD / (src.stem + '.o')
         if not force and obj.exists() and obj.stat().st_mtime > max(src.stat().st_mtime, newest_header):
             return obj, ''
-        r = subprocess.run([NVCC, *FLAGS, *[f'-D{d}' for d in defines], '-c', str(src), '-o', str(obj)], capture_output=True, text=True)
+        r = subprocess.run([NVCC, *FLAGS, '-c', str(src), '-o', str(obj)], capture_output=True, text=True)
         if r.returncode != 0:
             raise RuntimeError(f'nvcc failed for {src.name}:\n{r.stdout}\n{r.stderr}')
         (BUILD / (src.stem + '.ptxas.txt')).write_text(r.stderr)

@@ -444,12 +444,9 @@ int launch_wgrad(float* grads, const uint8_t* stash, const uint8_t* gstash, int 
 
 }  // namespace nerf
 
-extern "C" size_t nerf_mlp_backward_pipe_workspace_bytes(void);   // mlp_bwd_pipe.cu: link rings + flags of the fused backward
-
 extern "C" size_t nerf_mlp_backward_workspace_bytes(int64_t n_samples) {
   const uint64_t n_tiles = (uint64_t)((n_samples + nerf::kTile - 1) / nerf::kTile);
-  const size_t gstash = (size_t)(nerf::grad_tile_bytes_total() * n_tiles);
-  return ((gstash + 1023) & ~size_t(1023)) + nerf_mlp_backward_pipe_workspace_bytes();
+  return (size_t)(nerf::grad_tile_bytes_total() * n_tiles);
 }
 
 static int run_backward(float* grads, const float* d_rgbsigma, const float* rgbsigma, const void* stash, void* workspace,
@@ -496,25 +493,9 @@ static int run_backward(float* grads, const float* d_rgbsigma, const float* rgbs
   return 0;
 }
 
-extern "C" int nerf_mlp_backward_pipe(float* grads, const float* d_rgbsigma, const float* rgbsigma, const void* stash, void* workspace,
-                                      const void* packed, const float* params, int n_rays, int n_samples, float grad_scale, void* stream);
-
-// The production backward is the two-kernel path (tile-major dgrad chain + layer-major wgrad).  The layer-stationary fused pipeline
-// (mlp_bwd_pipe.cu) computes the same gradients with half the HBM traffic but is, as measured in round 2, ring-depth-bound and
-// slower (DESIGN.md section 4b); it stays exported as nerf_mlp_backward_pipe and can be made the default with -DNERF_BWD_PIPE.
 extern "C" int nerf_mlp_backward(float* grads, const float* d_rgbsigma, const float* rgbsigma, const void* stash, void* workspace,
                                  const void* packed, const float* params, int n_rays, int n_samples, float grad_scale,
                                  void* stream) {
-#ifdef NERF_BWD_PIPE
-  return nerf_mlp_backward_pipe(grads, d_rgbsigma, rgbsigma, stash, workspace, packed, params, n_rays, n_samples, grad_scale, stream);
-#else
-  return run_backward(grads, d_rgbsigma, rgbsigma, stash, workspace, packed, params, n_rays, n_samples, grad_scale, stream, 3);
-#endif
-}
-
-extern "C" int nerf_mlp_backward_legacy(float* grads, const float* d_rgbsigma, const float* rgbsigma, const void* stash, void* workspace,
-                                        const void* packed, const float* params, int n_rays, int n_samples, float grad_scale,
-                                        void* stream) {
   return run_backward(grads, d_rgbsigma, rgbsigma, stash, workspace, packed, params, n_rays, n_samples, grad_scale, stream, 3);
 }
 

@@ -64,28 +64,16 @@ __constant__ Job c_jobs[kNumJobs] = {
     {seg(1, kStashG, 2, 128, 0), {seg(0, kGradHead, 1, 4, 0), none()}, L::kWC1, 128, L::kBC1, 1, 6},
     {seg(1, hx(7), 4, 256, 0), {seg(0, kGradHead, 1, 4, 0), none()}, L::kWS, 256, L::kBS, 2, 9},
 };
-// Residual jobs of the fused backward (mlp_bwd_pipe.cu keeps the eight 256 x 256 layers' gradients on chip): the encoding
-// columns of layers 0 and 5 and the colour head; 320 KB of operands per tile instead of 1,424 KB.  CTAs proportional to bytes.
-constexpr int kNumResidualJobs = 4;
-__constant__ Job c_jobs_res[kNumResidualJobs] = {
-    {seg(0, gl(0), 4, 256, 0), {seg(1, kStashEnc, 1, 63, 0), none()}, L::kW0, 63, L::kB0, 0, 37},
-    {seg(0, gl(5), 4, 256, 0), {seg(1, kStashEnc, 1, 63, 256), none()}, L::kW5, 319, -1, 0, 37},
-    {seg(0, kGradC0, 2, 128, 0), {seg(1, kStashF, 4, 256, 0), seg(1, kStashDir, 1, 27, 256)}, L::kWC0, 283, L::kBC0, 0, 52},
-    {seg(1, kStashG, 2, 128, 0), {seg(0, kGradHead, 1, 4, 0), none()}, L::kWC1, 128, L::kBC1, 1, 22},
-};
 }  // namespace wg
 
 __global__ void __launch_bounds__(wg::kThreads, 1) mlp_wgrad_kernel(float* __restrict__ grads, const uint8_t* __restrict__ stash,
-                                                                     const uint8_t* __restrict__ gstash, int n_tiles, float inv_scale,
-                                                                     int residual) {
+                                                                     const uint8_t* __restrict__ gstash, int n_tiles, float inv_scale) {
   using namespace wg;
   // ---- which (job, part) is this CTA? ----
-  const Job* __restrict__ table = residual ? c_jobs_res : c_jobs;
-  const int n_jobs = residual ? kNumResidualJobs : kNumJobs;
   int job_idx = 0, part = (int)blockIdx.x;
-  while (job_idx < n_jobs && part >= table[job_idx].ctas) part -= table[job_idx++].ctas;
-  if (job_idx >= n_jobs) return;
-  const Job& job = table[job_idx];
+  while (job_idx < kNumJobs && part >= c_jobs[job_idx].ctas) part -= c_jobs[job_idx++].ctas;
+  if (job_idx >= kNumJobs) return;
+  const Job& job = c_jobs[job_idx];
   const int parts = job.ctas;
   const int tile_lo = (int)((int64_t)n_tiles * part / parts), tile_hi = (int)((int64_t)n_tiles * (part + 1) / parts);
   const int n_steps = 2 * (tile_hi - tile_lo);  // half tiles
@@ -279,26 +267,17 @@ __global__ void __launch_bounds__(wg::kThreads, 1) mlp_wgrad_kernel(float* __res
   if (warp == 2) tmem_dealloc(tmem_base, 512);
 }
 
-static int launch_wgrad_table(float* grads, const uint8_t* stash, const uint8_t* gstash, int n_tiles, float inv_scale, int residual, cudaStream_t stream);
-
 int launch_wgrad(float* grads, const uint8_t* stash, const uint8_t* gstash, int n_tiles, float inv_scale, cudaStream_t stream) {
-  return launch_wgrad_table(grads, stash, gstash, n_tiles, inv_scale, 0, stream);
-}
-int launch_wgrad_residual(float* grads, const uint8_t* stash, const uint8_t* gstash, int n_tiles, float inv_scale, cudaStream_t stream) {
-  return launch_wgrad_table(grads, stash, gstash, n_tiles, inv_scale, 1, stream);
-}
-
-static int launch_wgrad_table(float* grads, const uint8_t* stash, const uint8_t* gstash, int n_tiles, float inv_scale, int residual, cudaStream_t stream) {
   static bool attr_set_dev[64] = {};  // the attribute is per device
-    int dev__ = 0;
-    cudaGetDevice(&dev__);
-    bool& attr_set = attr_set_dev[dev__ & 63];
+  int dev__ = 0;
+  cudaGetDevice(&dev__);
+  bool& attr_set = attr_set_dev[dev__ & 63];
   if (!attr_set) {
     cudaError_t e = cudaFuncSetAttribute(mlp_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wg::kSmemBytes);
     NERF_CHECK_ARG(e == cudaSuccess, "mlp_backward: cudaFuncSetAttribute(wgrad) failed: %s", cudaGetErrorString(e));
     attr_set = true;
   }
-  mlp_wgrad_kernel<<<kNumSMs, wg::kThreads, wg::kSmemBytes, stream>>>(grads, stash, gstash, n_tiles, inv_scale, residual);
+  mlp_wgrad_kernel<<<kNumSMs, wg::kThreads, wg::kSmemBytes, stream>>>(grads, stash, gstash, n_tiles, inv_scale);
   NERF_CHECK_LAUNCH("mlp_wgrad_kernel");
   return 0;
 }

@@ -197,26 +197,6 @@ def mlp_backward(grads_flat: torch.Tensor, d_rgbsigma: torch.Tensor, rgbsigma: t
           'nerf_mlp_backward')
 
 
-def mlp_backward_legacy(grads_flat: torch.Tensor, d_rgbsigma: torch.Tensor, rgbsigma: torch.Tensor, stash: torch.Tensor,
-                        workspace: torch.Tensor, packed: torch.Tensor, params_flat: torch.Tensor, n_rays: int, n_samples: int,
-                        grad_scale: float = 1.0) -> None:
-    """K4, previous two-kernel path (tile-major dgrad chain + layer-major wgrad); kept for A/B timing and as a cross-check."""
-    require_device(grads_flat)
-    check(load().nerf_mlp_backward_legacy(ptr(grads_flat), ptr(d_rgbsigma), ptr(rgbsigma), ptr(stash), ptr(workspace), ptr(packed),
-                                          ptr(params_flat), n_rays, n_samples, float(grad_scale), stream_ptr()),
-          'nerf_mlp_backward_legacy')
-
-
-def mlp_backward_pipe(grads_flat: torch.Tensor, d_rgbsigma: torch.Tensor, rgbsigma: torch.Tensor, stash: torch.Tensor,
-                      workspace: torch.Tensor, packed: torch.Tensor, params_flat: torch.Tensor, n_rays: int, n_samples: int,
-                      grad_scale: float = 1.0) -> None:
-    """K4, fused layer-stationary pipeline (csrc/mlp_bwd_pipe.cu): same gradients, dY never leaves the chip (experimental)."""
-    require_device(grads_flat)
-    check(load().nerf_mlp_backward_pipe(ptr(grads_flat), ptr(d_rgbsigma), ptr(rgbsigma), ptr(stash), ptr(workspace), ptr(packed),
-                                        ptr(params_flat), n_rays, n_samples, float(grad_scale), stream_ptr()),
-          'nerf_mlp_backward_pipe')
-
-
 def mlp_backward_dgrad(d_rgbsigma, rgbsigma, stash, workspace, packed, params_flat, n_rays: int, n_samples: int) -> None:
     """K4a only: fills ``workspace`` with the per-layer output gradients."""
     require_device(d_rgbsigma)

@@ -44,7 +44,8 @@ def test_abi_version_and_layout_queries_work_without_gpu(library):
     assert len(off) == 24 and total == 595848 and sum(size) == 595844      # 595,844 parameters per block (SURVEY A.6)
     assert all(o % 4 == 0 for o in off)
     assert lib.nerf_mlp_packed_bytes() >= 2 * 557696 * 2                   # forward + transposed (dgrad) fp16 images
-    assert lib.nerf_mlp_stash_bytes(128) > 0 and lib.nerf_mlp_backward_workspace_bytes(128) > 0
+    assert lib.nerf_mlp_stash_bytes(128) > 0
+    assert lib.nerf_mlp_backward_workspace_bytes(128) == 638976             # one 128-sample tile of the gradient stash (624 KB)
 
 
 def test_no_cpu_fallback(library):

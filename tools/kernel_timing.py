@@ -9,7 +9,7 @@ import torch
 sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
 from nerficg_b200 import _lib, ops, params  # noqa: E402
 
-if os.environ.get('NERF_B200_LIB'):  # development: time a variant build (csrc/build.py tag=...)
+if os.environ.get('NERF_B200_LIB'):  # development: time another build of the library
     _lib.LIB_PATH = Path(os.environ['NERF_B200_LIB']).resolve()
 
 DEV = 'cuda:0'

@@ -36,7 +36,7 @@ def main():
         f = re.sub(r'<\d+, \d+>', '<K, pad>', k)
         fam.setdefault(f, []).append((k, c))
     print(f'# SASS inventory of `nerficg_b200/libnerf_b200.so` (final round-2 build, `cuobjdump -sass`, sm_100a; `python tools/sass_inventory.py`)\n')
-    print('`UTCHMMA` = tcgen05.mma (last column: how many are `.2CTA` = cta_group::2 -- the chain kernels and the fused pipeline; wgrad is single-CTA), `LDTM` = tcgen05.ld, `UBLKCP` = cp.async.bulk')
+    print('`UTCHMMA` = tcgen05.mma (last column: how many are `.2CTA` = cta_group::2 -- the chain kernels; wgrad is single-CTA), `LDTM` = tcgen05.ld, `UBLKCP` = cp.async.bulk')
     print('(TMA 1-D bulk copy), `SYNCS` = mbarrier ops, `USETMAXREG` = setmaxnreg, `RED`/`ATOMG` = global reductions. K2 is instantiated per')
     print('(keys per lane, padded cdf length): the row shows the range over its instances.\n')
     print('| kernel | instances | SASS instr | ' + ' | '.join(COLS) + ' | of which UTCHMMA.2CTA |')

@@ -1,7 +1,8 @@
-"""Runs pytest or a script of this repository against a development variant of the library (tools/variants.py):
+"""Runs pytest or a script of this repository against another build of the library, e.g. one built from an older checkout
+for an A/B comparison:
 
-    python tools/with_variant.py nerficg_b200/libnerf_b200.<tag>.so pytest tests/test_mlp_gpu.py -m gpu -q
-    python tools/with_variant.py nerficg_b200/libnerf_b200.<tag>.so bench.py --steps 30 --warmup 5
+    python tools/with_variant.py path/to/libnerf_b200.so pytest tests/test_mlp_gpu.py -m gpu -q
+    python tools/with_variant.py path/to/libnerf_b200.so bench.py --steps 30 --warmup 5
 
 The product binding (nerficg_b200/_lib.py) has no override of its own: this wrapper repoints it before anything loads it.
 """
