@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <cstdint>
 #include <cstdio>
+#include <initializer_list>
 
 namespace nerf {
 
@@ -26,6 +27,23 @@ void set_error(const char* fmt, ...);  // api.cu
   } while (0)
 
 constexpr int kNumSMs = 148;
+constexpr int kMaxDevices = 64;
+
+// Raises the dynamic shared-memory limit of `kernels` to `bytes` on the current device.  The attribute is per device, so
+// `done` (one static array per call site) remembers the devices where it has been set.
+inline cudaError_t set_max_dynamic_smem_once(bool (&done)[kMaxDevices], std::initializer_list<const void*> kernels, uint32_t bytes) {
+  int dev = 0;
+  cudaGetDevice(&dev);
+  bool& set = done[dev & (kMaxDevices - 1)];
+  if (set) return cudaSuccess;
+  cudaError_t err = cudaSuccess;
+  for (const void* fn : kernels) {
+    const cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    if (e != cudaSuccess) err = e;
+  }
+  set = err == cudaSuccess;
+  return err;
+}
 
 // ---- flat parameter layout of one NeRFBlock (see include/nerf_b200.h) -----------------
 // offsets in floats; every tensor start is padded to a multiple of 4 floats.

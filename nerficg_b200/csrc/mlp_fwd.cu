@@ -1,65 +1,41 @@
 // mlp_fwd.cu -- K3: positional encoding + the 8x256 skip-connected NeRF MLP as ONE fused,
-// persistent, warp-specialised tcgen05 kernel.
+// persistent, warp-specialised tcgen05 kernel on a CTA pair (chain.cuh), walking the 10-stage chain of mlp_layout.cuh.
 //
-// Two CTAs on the two SMs of a TPC form a cluster and work as a cta_group::2 PAIR: each CTA owns 128 samples of
-// a 256-sample "group" per slot, and walks two groups ("slots" 0/1) through the whole 10-stage chain
-// (mlp_layout.cuh) without touching HBM in between:
-//   warp 0      weight producer: streams THIS CTA's HALF of every fp16 weight panel (pre-swizzled UMMA images,
-//               128 of the 256 neurons) from L2 into a shared-memory ring with 1-D bulk copies + mbarriers
-//   warp 1      leader CTA: MMA issuer -- the warp runs the loop uniformly and ONE elected lane issues
-//               tcgen05.mma.cta_group::2 (M=256, N=256, K=16): rows 0..127 from its own activation panels
-//               and TMEM, rows 128..255 from the peer's, B = the two CTAs' ring stages (one half each), so a
-//               weight byte is fetched once per 256 samples; completion is multicast to both CTAs' barriers.
-//               peer CTA: relay -- forwards "my half of ring stage s has landed" to the leader's barrier.
-//               accumulators live in TMEM (2 slots x 256 fp32 columns = all 512 columns, in each CTA)
-//   warp 2      TMEM allocator
-//   warps 4-11  epilogue of slot 0 \  tcgen05.ld accumulator -> +bias, ReLU -> fp16 -> swizzled
-//   warps 12-19 epilogue of slot 1 /  A-operand panels of the next stage (in place); the two slots
-//               ping-pong so one slot's epilogue overlaps the other slot's MMAs.  Each slot has EIGHT warps:
-//               warp w owns TMEM lane quarter w % 4 (hardware rule) and column half (w / 4) % 2, so two warps
-//               per scheduler work on one accumulator.  Measured with four warps per slot: the serial loop
-//               MMA (2 K cycles) -> epilogue (4 K cycles, one latency-bound warp per scheduler) -> MMA left the
-//               tensor pipe idle half of the time.
-// The density head (256->1) and the RGB head (128->3, sigmoid) are evaluated on CUDA cores inside
-// the epilogues of stages 7 and 9, so the kernel emits packed (r,g,b,sigma) per sample.
-// Training additionally stashes every operand image the backward needs (bulk stores from shared
-// memory, region-major, see mlp_layout.cuh) and per-layer ReLU bit masks.
+// What only the forward does: the epilogues of stages 0..8 add the bias, apply ReLU and write fp16 A operand panels of
+// the next stage; the density head (256->1) and the RGB head (128->3, sigmoid) are evaluated on CUDA cores inside the
+// epilogues of stages 7 and 9, so the kernel emits packed (r,g,b,sigma) per sample.  Training additionally stashes every
+// operand image the backward needs (bulk stores from shared memory, region-major, see mlp_layout.cuh) and per-layer ReLU
+// bit masks.
 //
 // Measured lessons baked into the structure (DESIGN.md "K3"):
-//   * one CTA per tile pair was weight-starved: 128 KB of weights per 128 samples and layer is 64 B/cycle/SM at
-//     tensor peak (18 TB/s chip-wide) and the MMA issuer spent 24-40 % of its time waiting for ring stages; the
-//     CTA pair halves both the L2 -> SM stream and the shared-memory reads of B;
-//   * the issuing warp must stay warp-uniform with elect.sync around the tcgen05 instructions: issued under
-//     `if (lane == 0)` every MMA was wrapped in a compiler-generated ELECT/BRA.U.ANY waterfall and cost ~190
-//     cycles of issue for 64 cycles of tensor work;
 //   * N = 256 per instruction halves the instruction count and the re-reads of the A operand;
 //   * the epilogue prefetches the next chunk's bias (and density weights) while it processes the
 //     current one and takes the registers the producer / MMA warps do not need (setmaxnreg).
-#include "common.cuh"
-#include "mlp_layout.cuh"
-#include "tc.cuh"
+#include "chain.cuh"
 #include "../../include/nerf_b200.h"
 
 namespace nerf {
 using namespace tc;
 
 namespace fwd {
-constexpr int kEpiThreadsPerSlot = 256;  // 8 warps: 4 TMEM lane quarters x 2 column halves
-constexpr int kThreads = 128 + 2 * kEpiThreadsPerSlot;
-// weight ring: 16 KB stages = one K panel (64 inputs) x this CTA's 128 output neurons (64 for the colour layer)
 constexpr int kRingStages = 4;
-constexpr uint32_t kRingStageBytes = kPanelBytes128;
 // shared memory map (offsets from the 1024-aligned base)
 constexpr uint32_t kSlotBytes = kActBytes + kPanelBytes128;  // act (4 panels) + enc (1 panel)
 constexpr uint32_t kOffRing = 2 * kSlotBytes;
-constexpr uint32_t kOffBars = kOffRing + kRingStages * kRingStageBytes;
+constexpr uint32_t kOffBars = kOffRing + kRingStages * chain::kRingStageBytes;
 constexpr uint32_t kOffBias = kOffBars + 256;             // [2 slots][256 floats]: the bias vector of the stage in flight
 constexpr uint32_t kSmemBytes = kOffBias + 2 * 1024;      // the dynamic window is 1024-byte aligned (checked at kernel entry)
 static_assert(kSmemBytes <= 232448, "shared memory budget exceeded");
-constexpr int kRegsEpilogue = 112, kRegsOther = 32;
-// setmaxnreg moves registers inside the CTA's OWN allocation (launch: 640 threads x 96): what the 128 producer / MMA threads
-// release (96 - 32 each = 8192) must cover what the 512 epilogue threads request (112 - 96 each = 8192), or the
-// increase blocks forever
+
+struct Stages {
+  static constexpr int kStages = kFwdStages, kRingStages = fwd::kRingStages;
+  static constexpr int kProfBase = 0;  // stall-counter slots 0..9
+  __device__ static constexpr int panels(int st) { return fwd_panels(st); }
+  // every stage but the two 5-panel ones (skip layer, colour layer).  Measured (profiles/r02_chain_kernel_experiments.txt):
+  // the issuer's W-full wait halves and its A-ready wait grows by almost as much -- the epilogue is the critical path --
+  // so the gain is 1-2 % (inference 0.674 -> 0.667 ms, training 1.051 -> 1.038).
+  __device__ static constexpr bool shared(int st) { return fwd_panels(st) <= kRingStages; }
+};
 }  // namespace fwd
 
 struct FwdParams {
@@ -76,7 +52,7 @@ struct FwdParams {
   int n_samples;    // S
   int64_t n_evals;  // n_rays * S
   int n_tiles;
-  unsigned long long* prof;  // optional stall counters (common.cuh NERF_TIMED), slots 0..9
+  unsigned long long* prof;  // optional stall counters (chain.cuh), slots 0..9 and 22..24
 };
 
 // ---- per-row input encoding ----------------------------------------------------------------
@@ -161,211 +137,58 @@ __device__ __forceinline__ uint32_t hidden16(const uint32_t (&v)[32], const floa
   return m;
 }
 
-template <bool kV>
-struct BoolTag {
-  static constexpr bool value = kV;
-};
-
 // kProf: the stall counters (nerf_debug_set_timing) are compiled into their own instantiation; in the production one the
 // compiler drops every clock read and accumulator (with a run-time flag only, ptxas kept the 64-bit accumulators in local
 // memory and their reloads showed up in ncu's hot list)
 template <bool kTrain, bool kProf>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) mlp_fwd_kernel(const FwdParams p) {
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(chain::kThreads, 1) mlp_fwd_kernel(const FwdParams p) {
   using namespace fwd;
   using L = ParamLayout;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   const uint32_t smem_base = smem_u32(smem_raw);
   if ((smem_base & 1023u) != 0) __trap();  // SWIZZLE_128B operands need 1024-byte alignment and there is no slack to re-align
-  const uint32_t bars = smem_base + kOffBars;
-  // barrier map (8 bytes each)
-  const uint32_t bar_w_full = bars;                       // [kRingStages]
-  const uint32_t bar_w_empty = bars + 8 * kRingStages;    // [kRingStages]
-  const uint32_t bar_w_peer = bars + 16 * kRingStages;    // [kRingStages] leader only: the peer's half of the stage has landed
-  const uint32_t bar_a_ready = bars + 24 * kRingStages;   // [2] leader only: operands of BOTH CTAs written + accumulators drained
-  const uint32_t bar_acc_ready = bar_a_ready + 16;        // [2] accumulator complete (multicast commit)
-  const uint32_t bar_bias = bar_acc_ready + 16;           // [2] the slot's bias vector of the next stage has landed
-  const uint32_t tmem_slot = bar_bias + 16;               // uint32: TMEM base address
-  const uint32_t rank = cluster_ctarank();                // 0 = leader
-
+  const chain::Bars bars(smem_base + kOffBars, kRingStages, true);
+  const uint32_t rank = cluster_ctarank();  // 0 = leader
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  // Shared weight stages: the two slots of a CTA walk the chain one stage apart, so the weight panels of stage st are needed
-  // by slot 0 and, one accumulator later, by slot 1. They are loaded ONCE; slot 1's MMAs release the ring stages (half the
-  // L2 -> SM weight stream). Only stages whose panels all fit in the ring can be shared (slot 0 holds them until slot 1 is
-  // done): every stage but the two 5-panel ones (skip layer, colour layer).
-  // Measured (profiles/r02_chain_kernel_experiments.txt): the issuer's W-full wait halves and its A-ready wait grows by almost
-  // as much -- the epilogue is the critical path -- so the gain is 1-2 % (inference 0.674 -> 0.667 ms, training 1.051 -> 1.038).
-  auto shared_stage = [&](int st) { return fwd_panels(st) <= kRingStages; };
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < kRingStages; ++i) {
-      mbar_init(bar_w_full + 8 * i, 1);
-      mbar_init(bar_w_empty + 8 * i, 1);
-      mbar_init(bar_w_peer + 8 * i, 1);
-    }
-    for (int s = 0; s < 2; ++s) {
-      mbar_init(bar_a_ready + 8 * s, 16);  // one arrival per epilogue warp of either CTA
-      mbar_init(bar_acc_ready + 8 * s, 1);
-      mbar_init(bar_bias + 8 * s, 1);
-    }
-    fence_barrier_init();
-  }
-  if (warp == 2) {
-    tmem_alloc2(tmem_slot, 512);
-    tmem_relinquish2();
-  }
-  tc_fence_before();
-  cluster_sync_all();  // barriers of both CTAs initialised before any remote arrive / multicast commit
-  tc_fence_after();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
-
-  // group = 256 samples = one tile per CTA of the pair; a cluster handles two groups (slots) per iteration
-  const int n_clusters = (int)gridDim.x / 2, cluster_id = (int)blockIdx.x / 2;
-  const int n_groups = (p.n_tiles + 1) / 2;
-  const int n_iters = ((n_groups + 1) / 2 + n_clusters - 1) / n_clusters;
-  auto group_of = [&](int it, int slot) { return (it * n_clusters + cluster_id) * 2 + slot; };
-  auto active = [&](int it, int slot) { return group_of(it, slot) < n_groups; };  // identical in both CTAs
+  const uint32_t tmem_base = chain::setup(bars, warp);
+  const chain::Schedule sch(p.n_tiles);
   const bool prof_on = kProf && p.prof != nullptr;
 
   if (warp < 4) {
-    setmaxnreg_dec<kRegsOther>();
+    setmaxnreg_dec<chain::kRegsOther>();
     if (warp == 0) {
-      // =============================== weight producer ===============================
-      // one ring stage per K panel: rows [128 * rank, +128) of the 256-neuron panels, [64 * rank, +64) of the
-      // 128-neuron colour-layer panels (the cta_group::2 MMA takes the other half from the peer's ring)
-      uint32_t stage = 0, phase = 0;
-      const uint64_t keep = l2_evict_last();
-      long long t_wait = 0;
-      const long long t_begin = prof_on ? clock64() : 0;
-      for (int it = 0; it < n_iters; ++it) {
-        for (int st = 0; st < kFwdStages; ++st) {
-          for (int slot = 0; slot < 2; ++slot) {
-            if (!active(it, slot)) continue;
-            if (slot == 1 && shared_stage(st)) continue;   // slot 1 re-uses the panels loaded for slot 0
-            const int first = fwd_first_panel(st), np = fwd_panels(st);
-            const uint32_t bytes = st == 9 ? kRingStageBytes / 2 : kRingStageBytes;  // colour layer: 64 of 128 neurons
-            for (int pp = 0; pp < np; ++pp) {
-              NERF_TIMED(prof_on, t_wait, mbar_wait(bar_w_empty + 8 * stage, phase ^ 1));
-              if (elect_one()) {
-                mbar_arrive_expect_tx(bar_w_full + 8 * stage, bytes);
-                bulk_g2s_hint(smem_base + kOffRing + stage * kRingStageBytes, p.packed + fwd_panel_offset(first + pp) + rank * bytes, bytes,
-                              bar_w_full + 8 * stage, keep);
-              }
-              __syncwarp();
-              if (++stage == kRingStages) {
-                stage = 0;
-                phase ^= 1;
-              }
-            }
-          }
-        }
-      }
-      if (prof_on && lane == 0) {
-        atomicAdd(p.prof + 3, (unsigned long long)t_wait);
-        atomicAdd(p.prof + 4, (unsigned long long)(clock64() - t_begin));
-      }
+      chain::producer<Stages>(sch, bars, smem_base + kOffRing, prof_on, p.prof, [&](int st, int pp) {
+        const uint32_t bytes = st == 9 ? chain::kRingStageBytes / 2 : chain::kRingStageBytes;  // colour layer: 64 of 128 neurons
+        return chain::Panel{p.packed + fwd_panel_offset(fwd_first_panel(st) + pp) + rank * bytes, bytes};
+      });
     } else if (warp == 1 && rank == 0) {
-      // =============================== MMA issuer (leader CTA) ===============================
-      uint32_t stage = 0, phase = 0;
-      uint32_t a_phase[2] = {0, 0};
       constexpr uint32_t idesc256 = make_idesc(256, 256, kF16, kF16, 0, 0);
       constexpr uint32_t idesc128 = make_idesc(256, 128, kF16, kF16, 0, 0);
-      long long t_a = 0, t_w = 0;
-      const long long t_begin = prof_on ? clock64() : 0;
-      for (int it = 0; it < n_iters; ++it) {
-        for (int st = 0; st < kFwdStages; ++st) {
-          const bool sh = shared_stage(st);
-          const bool both = active(it, 1);
-          const uint32_t stage0 = stage, phase0 = phase;
-          for (int slot = 0; slot < 2; ++slot) {
-            if (!active(it, slot)) continue;
-            if (sh && slot == 1) {   // replay the ring stages slot 0 has just used (their barriers are still in the same phase)
-              stage = stage0;
-              phase = phase0;
-            }
-            const bool release = !sh || slot == 1 || !both;
-            const uint32_t act = smem_base + slot * kSlotBytes;
-            const uint32_t enc = act + kActBytes;
-            const uint32_t d_tmem = tmem_base + slot * 256;
-            NERF_TIMED(prof_on, t_a, mbar_wait_cluster(bar_a_ready + 8 * slot, a_phase[slot]));
-            a_phase[slot] ^= 1;
-            tc_fence_after();
-            const int np = fwd_panels(st);
-            for (int pp = 0; pp < np; ++pp) {
-              NERF_TIMED(prof_on, t_w, mbar_wait(bar_w_full + 8 * stage, phase));
-              NERF_TIMED(prof_on, t_w, mbar_wait_cluster(bar_w_peer + 8 * stage, phase));
-              tc_fence_after();
-              if (elect_one()) {
-                // A: stage 0 reads the encoding panel; panel 4 of stages 5 / 9 is the encoding / direction panel
-                const uint64_t da = make_smem_desc((st == 0 || pp == 4) ? enc : act + pp * kPanelBytes128, 16u, kAtomBytes);
-                const uint64_t db = make_smem_desc(smem_base + kOffRing + stage * kRingStageBytes, 16u, kAtomBytes);
-                const uint32_t idesc = st == 9 ? idesc128 : idesc256;
-                const int ksteps = (st == 9 && pp == 4) ? 2 : 4;  // the direction encoding is 32 wide
+      chain::issuer<Stages>(sch, bars, smem_base + kOffRing, tmem_base, prof_on, p.prof,
+                            [&](int st, int slot, int pp, uint32_t d_tmem, uint64_t db) {
+        const uint32_t act = smem_base + slot * kSlotBytes;
+        const uint32_t enc = act + kActBytes;
+        // A: stage 0 reads the encoding panel; panel 4 of stages 5 / 9 is the encoding / direction panel
+        const uint64_t da = make_smem_desc((st == 0 || pp == 4) ? enc : act + pp * kPanelBytes128, 16u, kAtomBytes);
+        const uint32_t idesc = st == 9 ? idesc128 : idesc256;
+        const int ksteps = (st == 9 && pp == 4) ? 2 : 4;  // the direction encoding is 32 wide
 #pragma unroll
-                for (int ks = 0; ks < 4; ++ks)
-                  if (ks < ksteps) umma2(d_tmem, da + 2u * ks, db + 2u * ks, idesc, (pp | ks) != 0);
-                if (release) umma_commit2(bar_w_empty + 8 * stage, 3);
-                if (pp == np - 1) umma_commit2(bar_acc_ready + 8 * slot, 3);
-              }
-              __syncwarp();
-              if (++stage == kRingStages) {
-                stage = 0;
-                phase ^= 1;
-              }
-            }
-          }
-        }
-      }
-      if (prof_on && lane == 0) {
-        atomicAdd(p.prof + 0, (unsigned long long)t_a);
-        atomicAdd(p.prof + 1, (unsigned long long)t_w);
-        atomicAdd(p.prof + 2, (unsigned long long)(clock64() - t_begin));
-        atomicAdd(p.prof + 9, 1ull);
-      }
+        for (int ks = 0; ks < 4; ++ks)
+          if (ks < ksteps) umma2(d_tmem, da + 2u * ks, db + 2u * ks, idesc, (pp | ks) != 0);
+      });
     } else if (warp == 1) {
-      // =============================== relay (peer CTA) ===============================
-      // tells the leader's issuer that this CTA's half of ring stage s has landed (bulk copies can only signal a
-      // barrier of their own CTA, and mbarriers cannot be waited on remotely)
-      uint32_t stage = 0, phase = 0;
-      for (int it = 0; it < n_iters; ++it)
-        for (int st = 0; st < kFwdStages; ++st)
-          for (int slot = 0; slot < 2; ++slot) {
-            if (!active(it, slot)) continue;
-            if (slot == 1 && shared_stage(st)) continue;
-            const int np = fwd_panels(st);
-            for (int pp = 0; pp < np; ++pp) {
-              mbar_wait(bar_w_full + 8 * stage, phase);
-              if (elect_one()) mbar_arrive_cluster(mapa(bar_w_peer + 8 * stage, 0));
-              __syncwarp();
-              if (++stage == kRingStages) {
-                stage = 0;
-                phase ^= 1;
-              }
-            }
-          }
+      chain::relay<Stages>(sch, bars);
     }
   } else {
     // =============================== epilogue warps ===============================
-    setmaxnreg_inc<kRegsEpilogue>();
-    const int ew = warp - 4;                 // 0..15
-    const int slot = ew >> 3;
-    const int half = (ew >> 2) & 1;          // column half of the accumulator owned by this warp
-    const int wq = warp & 3;                 // TMEM lane quarter of this warp (hardware: warp id % 4)
-    const int row = wq * 32 + lane;          // row of the tile; the thread of the other half has the same row
-    const int tg = threadIdx.x - 128 - slot * kEpiThreadsPerSlot;  // 0..255 within the slot
-    uint32_t act = smem_base + slot * kSlotBytes;
-    uint32_t t_slot = tmem_base + slot * 256 + (static_cast<uint32_t>(wq * 32) << 16);
-    const uint32_t bar_id = 1 + slot;  // named barrier of this slot's eight warps
-    uint32_t row_off = (uint32_t)(row >> 3) * kAtomBytes + (uint32_t)(row & 7) * kPanelRowBytes;
-    uint32_t xr = (uint32_t)(row & 7) << 4;  // swizzle term of this row: 16-byte chunk ch lives at ((ch << 4) ^ xr)
-    // opaque to the optimiser: otherwise ptxas re-derives these from %cluster_ctaid / %tid inside every chunk
-    // (S2UR + 10 dependent integer ops on the critical path of the operand stores)
-    asm volatile("" : "+r"(act), "+r"(t_slot), "+r"(row_off), "+r"(xr));
+    setmaxnreg_inc<chain::kRegsEpilogue>();
+    const chain::Epilogue epi(warp, lane, smem_base, kSlotBytes, tmem_base, bars);
+    const int slot = epi.slot, half = epi.half, row = epi.row, tg = epi.tg;
+    const uint32_t act = epi.act, t_slot = epi.t_slot, row_off = epi.row_off, xr = epi.xr;
     const uint32_t enc = act + kActBytes;
-    const uint32_t t_acc = t_slot + 128 * half;                            // hidden stages: columns [128 * half, +128)
-    const uint32_t act_h = act + 2 * half * kPanelBytes128 + row_off;      // this row in the first of this half's two panels
+    const uint32_t t_acc = t_slot + 128 * half;  // hidden stages: columns [128 * half, +128)
     uint32_t acc_phase = 0, bias_phase = 0;
     const uint64_t n_tiles64 = (uint64_t)p.n_tiles;
-    const uint32_t a_ready_leader = mapa(bar_a_ready + 8 * slot, 0);  // both CTAs announce their operands to the leader
     const bool prof = prof_on && tg == 0 && slot == 0;
     // the bias vector of the stage in flight lives in shared memory (one buffer per slot): after the slot's warps have
     // finished a stage (and met at a barrier) one thread bulk-copies the next stage's vector, which lands long before
@@ -375,45 +198,31 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
     auto bias_fetch = [&](int stage) {  // one thread; stage 0..7 hidden, 8 feature, 9 colour layer 0
       const float* src = p.params + (stage < 8 ? L::hidden_b(stage) : (stage == 8 ? L::kBF : L::kBC0));
       const uint32_t bytes = stage == 9 ? 512u : 1024u;
-      mbar_arrive_expect_tx(bar_bias + 8 * slot, bytes);
-      bulk_g2s(bias_u32, src, bytes, bar_bias + 8 * slot);
+      mbar_arrive_expect_tx(bars.bias + 8 * slot, bytes);
+      bulk_g2s(bias_u32, src, bytes, bars.bias + 8 * slot);
     };
-    if (tg == 0 && active(0, slot)) bias_fetch(0);
+    if (tg == 0 && sch.active(0, slot)) bias_fetch(0);
     long long t_accw = 0, t_drain = 0, t_pro = 0, t_bias = 0, t_bar = 0, t_mask = 0;
     const long long t_begin = prof ? clock64() : 0;
 
-    for (int it = 0; it < n_iters; ++it) {
-      if (!active(it, slot)) break;
-      const int tile = group_of(it, slot) * 2 + (int)rank;
-      const bool tile_ok = tile < p.n_tiles;  // the last group may have no tile for the peer: it still takes part in the MMAs
+    for (int it = 0; it < sch.n_iters; ++it) {
+      if (!sch.active(it, slot)) break;
+      const int tile = sch.tile(it, slot, rank);
+      const bool tile_ok = tile < p.n_tiles;
       const long long t_tile = prof ? clock64() : 0;
       const int64_t e = (int64_t)tile * kTile + row;  // sample index
       const bool valid = tile_ok && e < p.n_evals;
       const int ray = valid ? (int)(e / p.n_samples) : 0;
 
-      // stash helper: one thread bulk-stores an image from shared memory after the slot's warps fenced their writes
-      auto stash_issue = [&](int region, uint32_t src, uint32_t bytes) {  // one thread, after the slot's warps fenced + met
-        if (tg == 0 && tile_ok) {
-          uint8_t* dst = p.stash + stash_region_offset(region, n_tiles64) + (uint64_t)tile * stash_region_tile_bytes(region);
-          bulk_s2g_hint(dst, src, bytes, l2_evict_first());
-          bulk_commit();
-        }
+      // training only: the activation stash images
+      auto stash_dst = [&](int region) {
+        return [&, region] { return p.stash + stash_region_offset(region, n_tiles64) + (uint64_t)tile * stash_region_tile_bytes(region); };
       };
       auto stash_store = [&](int region, uint32_t src, uint32_t bytes) {
-        if (kTrain) {
-          fence_proxy_async_smem();
-          named_bar_sync(bar_id, kEpiThreadsPerSlot);
-          stash_issue(region, src, bytes);
-        }
+        if (kTrain) epi.image_store(stash_dst(region), src, bytes, tile_ok);
       };
-      // before overwriting a buffer that may still be read by an in-flight bulk store
       auto stash_drain = [&]() {
-        if (kTrain) {
-          const long long t0 = prof ? clock64() : 0;
-          if (tg == 0) bulk_wait_read<0>();
-          named_bar_sync(bar_id, kEpiThreadsPerSlot);
-          if (prof) t_drain += clock64() - t0;
-        }
+        if (kTrain) epi.image_drain(prof, t_drain);
       };
 
       // ---------------- prologue: position encoding -> enc panel (each half writes its 32 of the 64 columns) ----------------
@@ -456,16 +265,13 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
         write_half_row(enc, row, half, vals);
       }
       stash_store(kStashEnc, enc, kPanelBytes128);
-      fence_proxy_async_smem();
-      tc_fence_before();
-      __syncwarp();  // one (possibly remote) arrival per warp: per-thread remote arrivals serialise on the leader's barrier
-      if (lane == 0) mbar_arrive_cluster(a_ready_leader);
+      epi.hand_off();
       if (prof) t_pro += clock64() - t_tile;
 
       // next tile's prologue inputs (depths and the ray of each sample) -> L2, issued two stages before this tile ends
       auto prefetch_next_tile = [&]() {
-        if (half == 0 && it + 1 < n_iters && active(it + 1, slot)) {
-          const int next = group_of(it + 1, slot) * 2 + (int)rank;
+        if (half == 0 && it + 1 < sch.n_iters && sch.active(it + 1, slot)) {
+          const int next = sch.tile(it + 1, slot, rank);
           const int64_t en = (int64_t)next * kTile + row;
           if (next < p.n_tiles && en < p.n_evals) {
             asm volatile("prefetch.global.L2 [%0];" ::"l"(p.z + en));
@@ -484,7 +290,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
       for (int st = 0; st < 9; ++st) {
         const bool relu = st < 8;
         if (st == 7) prefetch_next_tile();
-        NERF_TIMED(prof, t_accw, mbar_wait(bar_acc_ready + 8 * slot, acc_phase));
+        NERF_TIMED(prof, t_accw, mbar_wait(bars.acc_ready + 8 * slot, acc_phase));
         acc_phase ^= 1;
         tc_fence_after();
         uint32_t mw[4] = {0u, 0u, 0u, 0u};  // ReLU bits of this thread's four 32-column chunks
@@ -499,7 +305,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
           uint32_t va[32], vb[32];
           tmem_ld32(t_acc, va);
           stash_drain();  // the act image of the previous stage may still be being stored
-          NERF_TIMED(prof, t_bias, mbar_wait(bar_bias + 8 * slot, bias_phase));
+          NERF_TIMED(prof, t_bias, mbar_wait(bars.bias + 8 * slot, bias_phase));
           // The bias words of 16-column group g + 1 are loaded BEFORE the (asm volatile, "memory") stores of group g: the compiler
           // cannot move the LDS across them by itself, and ncu's source view showed the first FADD of every group waiting on it
           // (13 % of the epilogue warps' samples).  Measured (round 2, profiles/r02_chain_kernel_experiments.txt): training
@@ -512,7 +318,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
           load4(ba, 0);
 #pragma unroll
           for (int c = 0; c < 4; c += 2) {
-            const uint32_t pbase = act_h + (uint32_t)(c >> 1) * kPanelBytes128;
+            const uint32_t pbase = epi.act_h + (uint32_t)(c >> 1) * kPanelBytes128;
             tmem_ld_wait32(va);
             load4(bb, 2 * c + 1);
             mw[c] = hidden16<kDens, kTrain, 0>(va, wsp + 32 * c, relu, pbase, 0u, xr, dens, ba);
@@ -529,7 +335,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
             mw[c + 1] |= hidden16<kDens, kTrain, 16>(vb, wsp + 32 * (c + 1), relu, pbase, 64u, xr, dens, bb);
           }
         };
-        if (st == 7) run(BoolTag<true>{}); else run(BoolTag<false>{});
+        if (st == 7) run(chain::BoolTag<true>{}); else run(chain::BoolTag<false>{});
         bias_phase ^= 1;
         if (st == 8) {
           // direction encoding -> enc panel (the x encoding was last read by stage 5): 27 values in half 0, zeros beyond
@@ -549,12 +355,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
         }
         // operands are handed to the MMA issuer per warp BEFORE the slot's warps meet for the image store / bias refill
         // (measured in round 2: inference 0.689 -> 0.667 ms at 4096 x 192, training unchanged)
-        fence_proxy_async_smem();
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive_cluster(a_ready_leader);
-        NERF_TIMED(prof, t_bar, named_bar_sync(bar_id, kEpiThreadsPerSlot));
-        if (kTrain) stash_issue(st < 8 ? kStashH0 + st : kStashF, act, kActBytes);
+        epi.hand_off();
+        NERF_TIMED(prof, t_bar, epi.sync());
+        if (kTrain) {
+          const int region = st < 8 ? kStashH0 + st : kStashF;
+          epi.image_issue(stash_dst(region), act, kActBytes, tile_ok);
+        }
         if (tg == 0) bias_fetch(st + 1);
         // ReLU bits -> stash, after the hand-off: a plain global store can stall its warp under the stash's HBM write load
         if (kTrain && relu && tile_ok) {
@@ -570,11 +376,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
         const int cb = 64 * half;  // this thread's 64 of the 128 colour-layer neurons
         float a0 = 0.f, a1 = 0.f, a2 = 0.f;
         uint32_t gm0 = 0u, gm1 = 0u;  // ReLU bits of this thread's two 32-column chunks of g
-        NERF_TIMED(prof, t_accw, mbar_wait(bar_acc_ready + 8 * slot, acc_phase));
+        NERF_TIMED(prof, t_accw, mbar_wait(bars.acc_ready + 8 * slot, acc_phase));
         acc_phase ^= 1;
         tc_fence_after();
         stash_drain();  // the F image store reads act, which receives g (and the partial sums) below
-        mbar_wait(bar_bias + 8 * slot, bias_phase);
+        mbar_wait(bars.bias + 8 * slot, bias_phase);
         bias_phase ^= 1;
 #pragma unroll 1
         for (int s = 0; s < 4; ++s) {
@@ -620,9 +426,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
         stash_store(kStashG, act, 2 * kPanelBytes128);  // (training) its barrier also orders the exchange
         if (!kTrain) {
           fence_proxy_async_smem();
-          named_bar_sync(bar_id, kEpiThreadsPerSlot);
+          epi.sync();
         }
-        if (tg == 0 && it + 1 < n_iters && active(it + 1, slot)) bias_fetch(0);  // first stage of this slot's next tile
+        if (tg == 0 && it + 1 < sch.n_iters && sch.active(it + 1, slot)) bias_fetch(0);  // first stage of this slot's next tile
         if (half == 0 && valid) {
           uint32_t r0, r1, r2, r3;
           asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3) : "r"(xch));
@@ -644,18 +450,13 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(fwd::kThreads, 1) ml
     }
     if (kTrain && tg == 0) bulk_wait_all<0>();
     if (prof) {
-      atomicAdd(p.prof + 5, (unsigned long long)t_accw);
-      atomicAdd(p.prof + 6, (unsigned long long)(clock64() - t_begin));
-      atomicAdd(p.prof + 7, (unsigned long long)t_drain);
-      atomicAdd(p.prof + 8, (unsigned long long)t_pro);
+      chain::epilogue_counters<Stages>(p.prof, t_accw, t_begin, t_drain, t_pro);
       atomicAdd(p.prof + 22, (unsigned long long)t_bias);   // (slots 10..21 belong to dgrad) waits the table above counts as busy time
       atomicAdd(p.prof + 23, (unsigned long long)t_bar);
       atomicAdd(p.prof + 24, (unsigned long long)t_mask);
     }
   }
-  tc_fence_before();
-  cluster_sync_all();  // the peer may still be reading this CTA's shared memory / arriving on its barriers
-  if (warp == 2) tmem_dealloc2(tmem_base, 512);
+  chain::teardown(tmem_base, warp);
 }
 
 }  // namespace nerf
@@ -693,30 +494,20 @@ extern "C" int nerf_mlp_forward(float* rgbsigma, void* stash, const void* packed
   p.n_evals = n_evals;
   p.n_tiles = (int)((n_evals + kTile - 1) / kTile);
   p.prof = reinterpret_cast<unsigned long long*>(timing_buffer());
-  const int group_pairs = ((p.n_tiles + 1) / 2 + 1) / 2;  // one cluster iteration = 2 slots x 2 tiles
-  const int grid = 2 * (group_pairs < kNumSMs / 2 ? group_pairs : kNumSMs / 2);
-  static bool attr_set_dev[64] = {};  // the attribute is per device
-    int dev__ = 0;
-    cudaGetDevice(&dev__);
-    bool& attr_set = attr_set_dev[dev__ & 63];
-  if (!attr_set) {
-    cudaError_t e1 = cudaSuccess;
-    for (auto fn : {(const void*)mlp_fwd_kernel<false, false>, (const void*)mlp_fwd_kernel<true, false>, (const void*)mlp_fwd_kernel<false, true>,
-                    (const void*)mlp_fwd_kernel<true, true>}) {
-      const cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fwd::kSmemBytes);
-      if (e != cudaSuccess) e1 = e;
-    }
-    NERF_CHECK_ARG(e1 == cudaSuccess, "mlp_forward: cudaFuncSetAttribute failed: %s", cudaGetErrorString(e1));
-    attr_set = true;
-  }
+  const int grid = chain::grid(p.n_tiles);
+  static bool smem_set[kMaxDevices] = {};
+  const cudaError_t e = set_max_dynamic_smem_once(
+      smem_set, {(const void*)mlp_fwd_kernel<false, false>, (const void*)mlp_fwd_kernel<true, false>,
+                 (const void*)mlp_fwd_kernel<false, true>, (const void*)mlp_fwd_kernel<true, true>}, fwd::kSmemBytes);
+  NERF_CHECK_ARG(e == cudaSuccess, "mlp_forward: cudaFuncSetAttribute failed: %s", cudaGetErrorString(e));
   const cudaStream_t st = static_cast<cudaStream_t>(stream);
   const bool with_prof = p.prof != nullptr;
   if (stash != nullptr) {
-    if (with_prof) mlp_fwd_kernel<true, true><<<grid, fwd::kThreads, fwd::kSmemBytes, st>>>(p);
-    else mlp_fwd_kernel<true, false><<<grid, fwd::kThreads, fwd::kSmemBytes, st>>>(p);
+    if (with_prof) mlp_fwd_kernel<true, true><<<grid, chain::kThreads, fwd::kSmemBytes, st>>>(p);
+    else mlp_fwd_kernel<true, false><<<grid, chain::kThreads, fwd::kSmemBytes, st>>>(p);
   } else {
-    if (with_prof) mlp_fwd_kernel<false, true><<<grid, fwd::kThreads, fwd::kSmemBytes, st>>>(p);
-    else mlp_fwd_kernel<false, false><<<grid, fwd::kThreads, fwd::kSmemBytes, st>>>(p);
+    if (with_prof) mlp_fwd_kernel<false, true><<<grid, chain::kThreads, fwd::kSmemBytes, st>>>(p);
+    else mlp_fwd_kernel<false, false><<<grid, chain::kThreads, fwd::kSmemBytes, st>>>(p);
   }
   NERF_CHECK_LAUNCH("mlp_fwd_kernel");
   return 0;

@@ -268,15 +268,9 @@ __global__ void __launch_bounds__(wg::kThreads, 1) mlp_wgrad_kernel(float* __res
 }
 
 int launch_wgrad(float* grads, const uint8_t* stash, const uint8_t* gstash, int n_tiles, float inv_scale, cudaStream_t stream) {
-  static bool attr_set_dev[64] = {};  // the attribute is per device
-  int dev__ = 0;
-  cudaGetDevice(&dev__);
-  bool& attr_set = attr_set_dev[dev__ & 63];
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(mlp_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wg::kSmemBytes);
-    NERF_CHECK_ARG(e == cudaSuccess, "mlp_backward: cudaFuncSetAttribute(wgrad) failed: %s", cudaGetErrorString(e));
-    attr_set = true;
-  }
+  static bool smem_set[kMaxDevices] = {};
+  const cudaError_t e = set_max_dynamic_smem_once(smem_set, {(const void*)mlp_wgrad_kernel}, wg::kSmemBytes);
+  NERF_CHECK_ARG(e == cudaSuccess, "mlp_backward: cudaFuncSetAttribute(wgrad) failed: %s", cudaGetErrorString(e));
   mlp_wgrad_kernel<<<kNumSMs, wg::kThreads, wg::kSmemBytes, stream>>>(grads, stash, gstash, n_tiles, inv_scale);
   NERF_CHECK_LAUNCH("mlp_wgrad_kernel");
   return 0;

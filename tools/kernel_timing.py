@@ -77,8 +77,7 @@ def main():
     v = buf[20:22].tolist()
     n_cta = max(buf[19].item(), 1)
     print(f'    prologue: loads+arithmetic {v[0] / n_cta:12.0f} cyc/CTA, store drain {v[1] / n_cta:12.0f} cyc/CTA')
-    v = buf[25:27].tolist()
-    print(f'    epilogue wait mask words   {v[0] / n_cta:12.0f} cyc/CTA, slot barrier {v[1] / n_cta:12.0f} cyc/CTA')
+    print(f'    epilogue wait mask words   {buf[25].item() / n_cta:12.0f} cyc/CTA')
     for _ in range(3):
         ops.mlp_backward_wgrad(grads, stash, ws, n_rays, s, 1024.0)
     a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
