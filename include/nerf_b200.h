@@ -112,6 +112,15 @@ int nerf_mlp_backward_dgrad(const float* d_rgbsigma, const float* rgbsigma, cons
 int nerf_mlp_backward_wgrad(float* grads, const void* stash, const void* workspace, int n_rays, int n_samples,
                             float grad_scale, void* stream);
 
+/* ---- K4c: gradients of NeRFBlock.forward w.r.t. its inputs ------------------------------
+ * Reads the `workspace` that nerf_mlp_backward_dgrad (or nerf_mlp_backward) filled for the same n_samples, with the
+ * samples laid out as in K3 with S = 1: sample e is the point positions[e] seen from directions[e] ([n_samples][3]).
+ * Writes d_positions / d_directions [n_samples][3] = dL/d(position, direction) after division by grad_scale (the scale
+ * the dgrad input was multiplied by).  Either output may be NULL and is then skipped; n_samples == 0 is a no-op. */
+int nerf_mlp_backward_inputs(float* d_positions, float* d_directions, const void* workspace, const float* params,
+                             const float* positions, const float* directions, int64_t n_samples, float grad_scale,
+                             void* stream);
+
 /* ---- K7: Adam on a flat parameter buffer (torch.optim.Adam semantics: no weight decay, no amsgrad) ----------
  * reference: src/Methods/NeRF/Trainer.py:32-37,61-63.  `state` = 4 device floats {step, 1-beta1^step,
  * sqrt(1-beta2^step), unused}; nerf_adam_tick advances it once per optimiser step (graph-replay safe), then

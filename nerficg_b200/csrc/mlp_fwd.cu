@@ -12,6 +12,7 @@
 //   * the epilogue prefetches the next chunk's bias (and density weights) while it processes the
 //     current one and takes the registers the producer / MMA warps do not need (setmaxnreg).
 #include "chain.cuh"
+#include "encoding.cuh"
 #include "../../include/nerf_b200.h"
 
 namespace nerf {
@@ -56,26 +57,7 @@ struct FwdParams {
 };
 
 // ---- per-row input encoding ----------------------------------------------------------------
-// 63 position features [x, cos(2^k x_i), sin(2^k x_i)] (reference utils.py:32-36) as 64 halves.
-// sin/cos of 2^k x are produced by exact sincosf at k = 0 and k = 5 plus double-angle steps
-// (<= 4 doublings: error <= 16 ulp, far below the fp16 operand rounding).
-__device__ __forceinline__ void encode_axis(float v, int n_freq, float* cs_out /* [2*n_freq]: cos block, sin block */) {
-  float s, c;
-#pragma unroll
-  for (int k = 0; k < 10; ++k) {
-    if (k >= n_freq) break;
-    if (k == 0 || k == 5) {
-      sincosf(v * (float)(1 << k), &s, &c);
-    } else {
-      const float s2 = 2.f * s * c;
-      const float c2 = 1.f - 2.f * s * s;
-      s = s2;
-      c = c2;
-    }
-    cs_out[k] = c;
-    cs_out[n_freq + k] = s;
-  }
-}
+// 63 position features [x, cos(2^k x_i), sin(2^k x_i)] (reference utils.py:32-36) as 64 halves (encode_axis: encoding.cuh).
 
 // chunks [4 * half, 4 * half + 4) of one panel row: 32 values -> 32 halves (each column half of a row has its own thread)
 __device__ __forceinline__ void write_half_row(uint32_t panel_smem, int row, int half, const float* vals /*[32]*/) {

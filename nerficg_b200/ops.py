@@ -211,6 +211,23 @@ def mlp_backward_wgrad(grads_flat, stash, workspace, n_rays: int, n_samples: int
                                          stream_ptr()), 'nerf_mlp_backward_wgrad')
 
 
+def mlp_backward_inputs(workspace: torch.Tensor, params_flat: torch.Tensor, positions: torch.Tensor | None,
+                        directions: torch.Tensor | None, n_samples: int, grad_scale: float = 1.0):
+    """K4c -- (dL/dpositions, dL/ddirections), each (n_samples, 3), from the ``workspace`` that K4a filled for the same
+    samples (S = 1).  Pass None for an input whose gradient is not wanted; its result is None."""
+    positions, directions = _f32c(positions), _f32c(directions)
+    require_device(workspace)
+    for t in (positions, directions):
+        if t is not None and tuple(t.shape) != (n_samples, 3):
+            raise ValueError(f'expected ({n_samples}, 3) inputs, got {tuple(t.shape)}')
+    d_pos = torch.empty((n_samples, 3), dtype=torch.float32, device=workspace.device) if positions is not None else None
+    d_dir = torch.empty((n_samples, 3), dtype=torch.float32, device=workspace.device) if directions is not None else None
+    check(load().nerf_mlp_backward_inputs(ptr(d_pos), ptr(d_dir), ptr(workspace), ptr(params_flat), ptr(positions),
+                                          ptr(directions), n_samples, float(grad_scale), stream_ptr()),
+          'nerf_mlp_backward_inputs')
+    return d_pos, d_dir
+
+
 def selftest_umma(a: torch.Tensor, b: torch.Tensor, mode: int) -> torch.Tensor:
     """D = A @ B^T on one 128-row tile through tcgen05 (tests only)."""
     a, b = _f32c(a), _f32c(b)
