@@ -121,6 +121,20 @@ int nerf_mlp_backward_inputs(float* d_positions, float* d_directions, const void
                              const float* positions, const float* directions, int64_t n_samples, float grad_scale,
                              void* stream);
 
+/* ---- K4r: gradients of render_rays w.r.t. its rays ---------------------------------------
+ * After nerf_mlp_backward(_dgrad) filled `workspace` for one pass (n_rays x n_samples samples at depths z [n_rays][S],
+ * laid out as in K3) and K6 produced d_rgbsigma for it (relu_mask = 1, grad_scale), ACCUMULATES
+ * dL/d(origins, dirs, viewdirs) [n_rays][3] / grad_scale of that pass into the three outputs (each may be NULL: skipped).
+ * dL/ddirs includes the compositing term d / |d|^2 * sum_s sigma_s dL/dsigma_s (interval lengths scale with |d|).
+ * `scratch` needs nerf_mlp_backward_rays_scratch_bytes(n_rays, n_samples) bytes and need not be initialised.
+ * Deterministic (no float atomics).  n_rays == 0 or all outputs NULL: no-op.  Invalid arguments return an error before
+ * any launch. */
+size_t nerf_mlp_backward_rays_scratch_bytes(int n_rays, int n_samples);
+int nerf_mlp_backward_rays(float* d_origins, float* d_dirs, float* d_viewdirs, void* scratch, const void* workspace,
+                           const float* params, const float* origins, const float* dirs, const float* viewdirs,
+                           const float* z, const float* rgbsigma, const float* d_rgbsigma, int n_rays, int n_samples,
+                           float grad_scale, void* stream);
+
 /* ---- K7: Adam on a flat parameter buffer (torch.optim.Adam semantics: no weight decay, no amsgrad) ----------
  * reference: src/Methods/NeRF/Trainer.py:32-37,61-63.  `state` = 4 device floats {step, 1-beta1^step,
  * sqrt(1-beta2^step), unused}; nerf_adam_tick advances it once per optimiser step (graph-replay safe), then

@@ -68,16 +68,18 @@ class RayBatch:
 
     def _gather(self, ids: torch.Tensor) -> 'RayBatch':
         """Index-tensor selection through ONE `nerf_gather_rays` launch for the five fields of the training batch
-        (reference RayBatch.__getitem__, Datasets/utils.py:598-613, is one torch gather per field)."""
+        (reference RayBatch.__getitem__, Datasets/utils.py:598-613, is one torch gather per field).  A field that requires
+        grad, while grad is enabled, is gathered by torch indexing so that gradients flow back into it."""
         from .. import ops
         n = ids.numel()
         src, dst, out = {}, {}, {}
+        grad_enabled = torch.is_grad_enabled()
         for k in self._FIELDS:
             t = getattr(self, k)
             if t is None:
                 out[k] = None
             elif k in self._GATHERED and t.dtype == torch.float32 and t.is_contiguous() and t.dim() == 2 and \
-                    t.shape[1] == (1 if k == 'alpha' else 3):
+                    t.shape[1] == (1 if k == 'alpha' else 3) and not (grad_enabled and t.requires_grad):
                 src[k] = t
                 dst[k] = out[k] = torch.empty((n, t.shape[1]), dtype=torch.float32, device=t.device)
             else:

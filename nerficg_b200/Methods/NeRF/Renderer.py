@@ -5,8 +5,11 @@ Per chunk of at most RAY_BATCH_SIZE rays (Renderer.py:45-47) the pipeline is
     K1 stratified depths -> K3 coarse MLP -> K5 composite (+weights) -> K2 inverse-CDF + merge
     -> K3 fine MLP -> K5 composite
 with the same torch RNG draws in the same order as the reference (rand(n,Nc), [randn coarse noise],
-rand(n,Nf), [randn fine noise]).  Differentiation w.r.t. the model parameters goes through ONE
-autograd node per chunk whose backward runs K6 (compositing backward) and K4 (MLP backward).
+rand(n,Nf), [randn fine noise]).  Differentiation goes through ONE autograd node per chunk whose backward runs, per
+pass, K6 (compositing backward), then K4 (MLP dgrad + wgrad) when a parameter needs grad or K4a (dgrad only) when none
+does, then K4r when a ray tensor needs grad: dL/d(origin, direction, view_direction) reduced per ray from the same
+gradient stash (d also gets the compositing term, the interval lengths scale with |d|).  Without a ray tensor that
+requires grad the backward is exactly the parameter-only one.
 """
 from __future__ import annotations
 
@@ -86,7 +89,7 @@ class _RenderChunk(torch.autograd.Function):
         with stage('K5 composite fine'):
             rgb, depth, alpha, _ = ops.composite_forward(z, rs_f, direction, st.background)
         if need:
-            ctx.saved = (direction, z_c, rs_c, stash_c, z, rs_f, stash_f)
+            ctx.saved = (origin, direction, view_direction, z_c, rs_c, stash_c, z, rs_f, stash_f)
         return (rgb, depth, alpha, *outs)
 
     @staticmethod
@@ -95,29 +98,43 @@ class _RenderChunk(torch.autograd.Function):
         n_blocks = 2 if st.n_coarse > 0 else 1
         if not st.need_grad:
             return (None,) * (8 + 24 * n_blocks)
-        direction, z_c, rs_c, stash_c, z, rs_f, stash_f = ctx.saved
+        origin, direction, view_direction, z_c, rs_c, stash_c, z, rs_f, stash_f = ctx.saved
         n = z.shape[0]
         scale = default_grad_scale(n)
         ws = _Workspace.get(z.device, ops.mlp_backward_workspace_bytes(z.numel()))
+        need_params = any(ctx.needs_input_grad[8:])
+        # dL/d(origin, direction, view_direction): both passes add into these
+        d_rays = [torch.zeros(n, 3, device=z.device) if need else None for need in ctx.needs_input_grad[1:4]]
+        need_rays = any(t is not None for t in d_rays)
 
         def one(flat, packed, zz, rs, stash, gr, gd, ga):
-            grad = torch.zeros_like(flat)
+            grad = torch.zeros_like(flat) if need_params else None
             if gr is None and gd is None and ga is None:
                 return grad
             gr = torch.zeros(n, 3, device=zz.device) if gr is None else gr
             flatten = lambda t: None if t is None else t.reshape(-1)
             with stage('K6 composite_bwd'):
                 d_rs = ops.composite_backward(zz, rs, direction, st.background, gr, flatten(gd), flatten(ga), True, scale)
-            with stage('K4 mlp_bwd (dgrad + wgrad)'):
-                ops.mlp_backward(grad, d_rs, rs, stash, ws, packed, flat, n, zz.shape[1], scale)
+            if need_params:
+                with stage('K4 mlp_bwd (dgrad + wgrad)'):
+                    ops.mlp_backward(grad, d_rs, rs, stash, ws, packed, flat, n, zz.shape[1], scale)
+            else:
+                with stage('K4a mlp_bwd dgrad'):
+                    ops.mlp_backward_dgrad(d_rs, rs, stash, ws, packed, flat, n, zz.shape[1])
+            if need_rays:  # before the next pass's dgrad overwrites ws
+                with stage('K4r mlp_bwd rays'):
+                    ops.mlp_backward_rays(*d_rays, ws, flat, origin, direction, view_direction, zz, rs, d_rs, scale)
             return grad
+
+        def param_grads(grad):
+            return [None] * 24 if grad is None else list(params.views(grad).values())
 
         grads = []
         if st.n_coarse > 0:
-            grads += list(params.views(one(st.flat_c, st.packed_c, z_c, rs_c, stash_c, g_rgb_c, g_depth_c, g_alpha_c)).values())
-        grads += list(params.views(one(st.flat_f, st.packed_f, z, rs_f, stash_f, g_rgb, g_depth, g_alpha)).values())
+            grads += param_grads(one(st.flat_c, st.packed_c, z_c, rs_c, stash_c, g_rgb_c, g_depth_c, g_alpha_c))
+        grads += param_grads(one(st.flat_f, st.packed_f, z, rs_f, stash_f, g_rgb, g_depth, g_alpha))
         ctx.saved = None
-        return (None,) * 8 + tuple(grads)
+        return (None, *d_rays) + (None,) * 4 + tuple(grads)
 
 
 class NeRFRayRenderingComponent(BaseRenderingComponent):
@@ -141,7 +158,10 @@ class NeRFRayRenderingComponent(BaseRenderingComponent):
         st.n_coarse, st.n_fine = n_samples_coarse_nerf, n_samples_nerf
         blocks = ([self.coarse_nerf] if use_coarse else []) + [self.nerf]
         model_params = [p for b in blocks for p in b.ordered_parameters()]
-        st.need_grad = torch.is_grad_enabled() and any(p.requires_grad for p in model_params)
+        # stashes (and the backward weight images) are kept when a parameter or a ray tensor needs grad
+        ray_tensors = (rays.origin, rays.direction, rays.view_direction)
+        st.need_grad = torch.is_grad_enabled() and (any(p.requires_grad for p in model_params)
+                                                    or any(t is not None and t.requires_grad for t in ray_tensors))
         st.flat_f = self.nerf.flat_params
         st.flat_c = self.coarse_nerf.flat_params if use_coarse else None
         # weight images are rebuilt on every call (15 us per block): parameters may have changed in place

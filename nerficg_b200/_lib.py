@@ -32,6 +32,8 @@ _PROTOTYPES = {
     'nerf_mlp_backward_dgrad': (c_int, [c_void_p] * 6 + [c_int, c_int, c_void_p]),
     'nerf_mlp_backward_wgrad': (c_int, [c_void_p] * 3 + [c_int, c_int, c_float, c_void_p]),
     'nerf_mlp_backward_inputs': (c_int, [c_void_p] * 6 + [c_int64, c_float, c_void_p]),
+    'nerf_mlp_backward_rays_scratch_bytes': (c_size_t, [c_int, c_int]),
+    'nerf_mlp_backward_rays': (c_int, [c_void_p] * 12 + [c_int, c_int, c_float, c_void_p]),
     'nerf_adam_tick': (c_int, [c_void_p, c_float, c_float, c_void_p]),
     'nerf_adam_update': (c_int, [c_void_p] * 6 + [c_float, c_float, c_float, c_int64, c_void_p]),
     'nerf_adam_update_ex': (c_int, [c_void_p] * 6 + [c_float, c_float, c_float, c_float, c_int, c_int64, c_void_p]),

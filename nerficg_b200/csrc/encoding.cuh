@@ -26,4 +26,8 @@ __device__ __forceinline__ void encode_axis(float v, int n_freq, float* cs_out /
   }
 }
 
+// Coordinate of the sample at depth z on the ray o + d z, rounded as K3 rounds it (no fused multiply-add): the input
+// gradients differentiate cos / sin of 2^9 x, so they must see the forward's x to the last bit.
+__device__ __forceinline__ float ray_point(float o, float d, float z) { return __fadd_rn(o, __fmul_rn(d, z)); }
+
 }  // namespace nerf

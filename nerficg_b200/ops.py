@@ -228,6 +228,31 @@ def mlp_backward_inputs(workspace: torch.Tensor, params_flat: torch.Tensor, posi
     return d_pos, d_dir
 
 
+def mlp_backward_rays(d_origins: torch.Tensor | None, d_dirs: torch.Tensor | None, d_viewdirs: torch.Tensor | None,
+                      workspace: torch.Tensor, params_flat: torch.Tensor, origins, dirs, viewdirs, z, rgbsigma, d_rgbsigma,
+                      grad_scale: float = 1.0) -> None:
+    """K4r -- ACCUMULATES one pass's dL/d(origins, dirs, viewdirs) into the (n_rays, 3) fp32 tensors ``d_origins``,
+    ``d_dirs``, ``d_viewdirs`` (None: skipped), from the ``workspace`` K4a filled for the pass's samples at depths ``z``
+    (n_rays, S) and the ``d_rgbsigma`` K6 produced for it with ``grad_scale``.  The outputs are not zeroed here."""
+    origins, dirs, viewdirs, z = _f32c(origins), _f32c(dirs), _f32c(viewdirs), _f32c(z)
+    rgbsigma, d_rgbsigma = _f32c(rgbsigma), _f32c(d_rgbsigma)
+    require_device(workspace)
+    n, s = z.shape
+    for t in (d_origins, d_dirs, d_viewdirs, origins, dirs, viewdirs):
+        if t is not None and tuple(t.shape) != (n, 3):
+            raise ValueError(f'expected ({n}, 3) rays, got {tuple(t.shape)}')
+    for t in (d_origins, d_dirs, d_viewdirs):
+        if t is not None and (t.dtype != torch.float32 or not t.is_contiguous()):
+            raise TypeError('ray gradient accumulators must be contiguous float32')
+    for t in (rgbsigma, d_rgbsigma):
+        if t is not None and t.numel() != n * s * 4:
+            raise ValueError('rgbsigma and d_rgbsigma must hold 4 floats per sample')
+    scratch = torch.empty(int(load().nerf_mlp_backward_rays_scratch_bytes(n, s)), dtype=torch.uint8, device=workspace.device)
+    check(load().nerf_mlp_backward_rays(ptr(d_origins), ptr(d_dirs), ptr(d_viewdirs), ptr(scratch), ptr(workspace),
+                                        ptr(params_flat), ptr(origins), ptr(dirs), ptr(viewdirs), ptr(z), ptr(rgbsigma),
+                                        ptr(d_rgbsigma), n, s, float(grad_scale), stream_ptr()), 'nerf_mlp_backward_rays')
+
+
 def selftest_umma(a: torch.Tensor, b: torch.Tensor, mode: int) -> torch.Tensor:
     """D = A @ B^T on one 128-row tile through tcgen05 (tests only)."""
     a, b = _f32c(a), _f32c(b)
